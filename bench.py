@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the fused MARL-nav environment step on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[3]): 1,048,576 parallel envs x 3 agents x 3
 obstacles per GPU, policy-like random actions (SURVEY.md section 8d: turn angle
@@ -29,6 +29,8 @@ One JSON line on stdout (rank 0):
 marlnav.environment.Env from baseline/_ref (vendored, git-ignored, by __graft_entry__.build())
 at the full batch size, all host threads; its line also carries ``reference_cuda`` -- the same
 unmodified Env on device='cuda' (BASELINE.md 4.4's second bar).
+--dump-outputs DIR writes what the last timed Env.step returned (see dump_outputs) so that two
+builds can be compared output for output: the inputs depend only on the arguments.
 """
 import argparse
 import json
@@ -376,6 +378,24 @@ def rollout_record(B, dev, T=250):
             "what": "RolloutGraph: {fused actor sample -> fused step} x T with the critic on a parallel branch, one graph launch per rollout"}
 
 
+def dump_outputs(path, result, seed=0, budget=48 << 20):
+    """Writes one Env.step result -- the six Observations fields, rewards, terminated, truncated --
+    as float32 DIR/<name>.npy, env rows first.  A batch larger than `budget` bytes is cut to a fixed,
+    seeded sample of env rows, the same rows in every array; env_index.npy (float64) lists them."""
+    import numpy as np
+    fields, rew, term, trunc = result
+    arrays = dict(fields._asdict(), rewards=rew, terminated=term, truncated=trunc)
+    B = rew.shape[0]
+    per_env = 4 * sum(t[0].numel() for t in arrays.values()) + 8
+    n = min(B, budget // per_env)
+    idx = np.arange(B) if n == B else np.sort(np.random.default_rng(seed).choice(B, n, replace=False))
+    rows = torch.from_numpy(idx).to(rew.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.index_select(0, rows).to(torch.float32).cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     import marlnav_b200 as mb
@@ -430,14 +450,18 @@ def run_ours(args):
         sampler.arm()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for i in range(K):
+    for i in range(K - 1):
         env.step(pool[i % 16])
+    last = env.step(pool[(K - 1) % 16])              # kept for --dump-outputs
     e1.record()
     sampler.arm()                                    # the GPU is still executing the K steps
     barrier()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
     stats_delta = env.episode_stats.clone() - stats0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     # the same loop writing into one reused output buffer (what the round-1 line timed)
     out = env._alloc_outputs()
     ms_fused = cuda_time(lambda i: env.step_fused(pool[i % 16], out=out), K) * K
@@ -571,7 +595,13 @@ def main():
                     help="turn-angle range of the random actions in rad (SURVEY 8d: 0.2 policy-like, 3.14159 trig stress)")
     ap.add_argument("--prewarm-s", type=float, default=0.5,
                     help="seconds of device copies before the warm-up steps (P-state ramp)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (rank 0's slice) to DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)
