@@ -289,4 +289,8 @@ const char* marlnav_rollout_last_error(void);
 #ifdef __cplusplus
 }
 #endif
+
+/* float16 / bfloat16 observations: the `_typed` entry points */
+#include "marlnav_b200_typed.h"
+
 #endif /* MARLNAV_B200_H */

@@ -21,6 +21,8 @@ EXPORTS = ("marlnav_abi_version", "marlnav_last_error", "marlnav_obs_size", "mar
            "marlnav_step_launch_info", "marlnav_actor_sample_f32", "marlnav_act_step_f32", "marlnav_critic_value_f32",
            "marlnav_discounted_returns_f64",
            "marlnav_rollout_last_error")
+# every symbol include/marlnav_b200_typed.h declares (16-bit observations; included by marlnav_b200.h)
+TYPED_EXPORTS = ("marlnav_observe_typed", "marlnav_step_typed", "marlnav_step_call_typed", "marlnav_step_host_typed")
 
 
 class _Sized(ctypes.Structure):
@@ -105,7 +107,7 @@ def load():
     lib.marlnav_rollout_last_error.restype = ctypes.c_char_p
     sizeofs = ("marlnav_sizeof_env_params", "marlnav_sizeof_reset_spec", "marlnav_sizeof_io_transform",
                "marlnav_sizeof_actor_spec", "marlnav_sizeof_step_call")
-    for name in EXPORTS:
+    for name in EXPORTS + TYPED_EXPORTS:
         if name in sizeofs:
             getattr(lib, name).restype = ctypes.c_size_t
         elif name == "marlnav_host_pipe_destroy":
@@ -118,6 +120,10 @@ def load():
     lib.marlnav_observe_f32.argtypes = [vp] * 6
     lib.marlnav_init_f32.argtypes = [vp] * 8
     lib.marlnav_step_host_f32.argtypes = [vp] * 21
+    lib.marlnav_observe_typed.argtypes = [vp] * 5 + [i32, vp]
+    lib.marlnav_step_typed.argtypes = [vp] * 9 + [i32] + [vp] * 6
+    lib.marlnav_step_call_typed.argtypes = [vp, i32]
+    lib.marlnav_step_host_typed.argtypes = [vp] * 21 + [i32]
     lib.marlnav_host_pipe_create.argtypes = [ctypes.POINTER(vp)]
     lib.marlnav_host_pipe_destroy.argtypes = [vp]
     lib.marlnav_act_step_f32.argtypes = [vp] * 18

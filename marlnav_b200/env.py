@@ -28,6 +28,10 @@ Differences from the reference, all documented in DESIGN.md:
     processes stepping N slices reproduce the single-process run bit for bit.
   * ``init_method='template'`` accepts an explicit (A,5) agent template for team
     sizes the reference's 3-agent triangle cannot express.
+  * ``params['obs_dtype']`` (default ``torch.float32``) may be ``torch.float16`` or
+    ``torch.bfloat16``: every observation the env returns is then the float32 value
+    rounded to nearest-even (``obs32.to(dtype)``, bit for bit); rewards, flags and the
+    state are unchanged.
 """
 import ctypes
 import math
@@ -55,6 +59,10 @@ def _triangle_agents(init):
     heading = torch.tensor([[1., 0.]] * 3)
     speed = init['init_speed'] * torch.ones(3, 1)
     return torch.cat([pos, heading, speed], dim=1)
+
+
+# observation element types: torch dtype -> MARLNAV_OBS_* code of the `_typed` entry points
+OBS_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
 
 
 def split_observations(obs, num_agents, num_obstacles):
@@ -93,6 +101,12 @@ class Env(object):
             raise _lib.MarlnavError(
                 f"unsupported team shape A={self.num_agents}, O={self.num_obstacles} "
                 "(need 2 <= A <= 26, 1 <= O <= 64)")
+        # fixed for the env's life: output slots, captured graphs and host buffers are sized from it
+        self.obs_dtype = params.get('obs_dtype', torch.float32)
+        if self.obs_dtype not in OBS_DTYPES:
+            raise _lib.MarlnavError(f"obs_dtype must be torch.float32, torch.float16 or torch.bfloat16, "
+                                    f"got {self.obs_dtype!r}")
+        self._obs_code = OBS_DTYPES[self.obs_dtype]
         self._sampler = action_sampler(params.get('sampler'))
         self._others_inds = torch.tensor(
             [[i for i in range(self.num_agents) if i != j] for j in range(self.num_agents)],
@@ -288,8 +302,9 @@ class Env(object):
         return self._sampler()
 
     def supports_fused_actor(self, actor):
-        """Is there a fused {actor -> step} kernel for this env and actor (marlnav_act_step_f32)?"""
-        return (self.num_agents == 3 and 1 <= self.num_obstacles <= 6 and self._io is not None
+        """Is there a fused {actor -> step} kernel for this env and actor (marlnav_act_step_f32)?
+        Not for 16-bit observations: the fused actor reads and writes float32."""
+        return (self.obs_dtype == torch.float32 and self.num_agents == 3 and 1 <= self.num_obstacles <= 6 and self._io is not None
                 and bool(self._io.obs_mean) and bool(self._io.act_scale)
                 and getattr(actor, 'obs_size', None) == self.obs_size and getattr(actor, 'hidden', 10 ** 9) <= 256
                 and getattr(getattr(actor, 'w1', None), 'device', None) == self.states.device)
@@ -298,7 +313,10 @@ class Env(object):
         """``actor.act(obs_in)`` + ``step_fused`` as ONE launch (SURVEY 8(f)-2; models.py:113-122).
         ``obs_in`` (B,A,S): the normalised observations of the current state; ``out`` = preallocated
         (actions (B*A,2), log_probs (B*A), next_obs (B,A,S), rewards (B), terminated_u8 (B),
-        truncated_u8 (B)).  Needs ``fuse_io`` with both transforms."""
+        truncated_u8 (B)).  Needs ``fuse_io`` with both transforms and float32 observations."""
+        if self.obs_dtype != torch.float32:
+            raise _lib.MarlnavError(f"act_step_fused reads and writes float32 observations; this env's obs_dtype "
+                                    f"is {self.obs_dtype}")
         if not self.supports_fused_actor(actor):
             raise _lib.MarlnavError("no fused actor+step kernel for this env/actor (see supports_fused_actor)")
         actions, log_probs, obs, rew, term, trunc = out
@@ -414,13 +432,18 @@ class Env(object):
         self.__dict__.pop('_call_cache', None)
 
     def observations_fused(self):
-        """(B,A,S) observation buffer of the current states (one kernel launch)."""
+        """(B,A,S) observation buffer of the current states, in ``obs_dtype`` (one kernel launch)."""
         B, A = self.num_parallel, self.num_agents
         with torch.cuda.device(self.device):
-            obs = torch.empty(B, A, self.obs_size, device=self.device)
-            _lib.check(self._lib.marlnav_observe_f32(
-                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
-                self._ptr(self.target), self._ptr(obs), self._stream()), "marlnav_observe_f32")
+            obs = torch.empty(B, A, self.obs_size, dtype=self.obs_dtype, device=self.device)
+            if self._obs_code == 0:
+                _lib.check(self._lib.marlnav_observe_f32(
+                    ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
+                    self._ptr(self.target), self._ptr(obs), self._stream()), "marlnav_observe_f32")
+            else:
+                _lib.check(self._lib.marlnav_observe_typed(
+                    ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
+                    self._ptr(self.target), self._ptr(obs), self._obs_code, self._stream()), "marlnav_observe_typed")
         return obs
 
     def observations(self):
@@ -429,11 +452,12 @@ class Env(object):
 
     def _alloc_outputs(self):
         B, A, S = self.num_parallel, self.num_agents, self.obs_size
-        n_obs = B * A * S * 4
+        n_obs_used = B * A * S * self.obs_dtype.itemsize
+        n_obs = (n_obs_used + 15) & ~15               # rewards and flags stay 16-byte aligned
         n_rew = (B * 4 + 15) & ~15
         n_flag = (B + 15) & ~15
         buf = torch.empty(n_obs + n_rew + 2 * n_flag, dtype=torch.uint8, device=self.device)
-        obs = buf[:n_obs].view(torch.float32).view(B, A, S)
+        obs = buf[:n_obs_used].view(self.obs_dtype).view(B, A, S)
         rew = buf[n_obs:n_obs + B * 4].view(torch.float32)
         term = buf[n_obs + n_rew:n_obs + n_rew + B]
         trunc = buf[n_obs + n_rew + n_flag:n_obs + n_rew + n_flag + B]
@@ -468,7 +492,12 @@ class Env(object):
         if c is None:
             rs = self._reset_spec(alias=False)
             self._call_epoch = self.__dict__.get('_call_epoch', 0) + 1
-            c = dict(rs=rs, epoch=self._call_epoch, fn=self._lib.marlnav_step_call_f32)
+            if self._obs_code == 0:
+                fn = self._lib.marlnav_step_call_f32
+            else:
+                typed, code = self._lib.marlnav_step_call_typed, self._obs_code
+                fn = lambda call: typed(call, code)
+            c = dict(rs=rs, epoch=self._call_epoch, fn=fn)
             self._call_cache = c
         return c
 
@@ -517,7 +546,7 @@ class Env(object):
         call.stream = stream
         rc = c['fn'](ctypes.addressof(call))
         if rc:
-            _lib.check(rc, "marlnav_step_call_f32")
+            _lib.check(rc, "marlnav_step_call_f32" if self._obs_code == 0 else "marlnav_step_call_typed")
         self._commit_step_counter()
         if self._alias_pending:
             # the reference's template froze at "state after the first move" (B-6)
@@ -528,9 +557,15 @@ class Env(object):
     def step_fused(self, actions, out=None):
         """One fused step.  Returns ``(obs (B,A,S), rewards (B), terminated (B) bool,
         truncated (B) bool)``; ``out`` may supply preallocated (obs, rewards,
-        terminated_u8, truncated_u8) tensors to write into."""
+        terminated_u8, truncated_u8) tensors to write into; ``obs`` must have the env's
+        ``obs_dtype`` and at least B*A*S elements."""
         if out is not None:
             obs, rew, term, trunc = out
+            if obs.dtype != self.obs_dtype or obs.numel() < self.num_parallel * self.num_agents * self.obs_size:
+                raise _lib.MarlnavError(
+                    f"step_fused: out[0] must be {self.obs_dtype} with at least "
+                    f"{self.num_parallel * self.num_agents * self.obs_size} elements, got {obs.dtype} "
+                    f"with {obs.numel()}")
             self._launch_step(actions, (obs.data_ptr(), rew.data_ptr(), term.data_ptr(), trunc.data_ptr()))
             return obs, rew, term.view(torch.bool), trunc.view(torch.bool)
         slot, stream = self._take_slot()
@@ -562,17 +597,17 @@ class HostStepper:
         B, A, S = env.num_parallel, env.num_agents, env.obs_size
         dev = env.device
         self.actions_host = torch.empty(B, A, 2, pin_memory=True)
-        self.obs_host = torch.empty(B, A, S, pin_memory=True)
+        self.obs_host = torch.empty(B, A, S, dtype=env.obs_dtype, pin_memory=True)
         self.rewards_host = torch.empty(B, pin_memory=True)
         self.terminated_host = torch.empty(B, dtype=torch.uint8, pin_memory=True)
         self.truncated_host = torch.empty(B, dtype=torch.uint8, pin_memory=True)
         self.actions_dev = torch.empty(B, A, 2, device=dev)
-        self.obs_dev = torch.empty(B, A, S, device=dev)
+        self.obs_dev = torch.empty(B, A, S, dtype=env.obs_dtype, device=dev)
         self.rewards_dev = torch.empty(B, device=dev)
         self.terminated_dev = torch.empty(B, dtype=torch.uint8, device=dev)
         self.truncated_dev = torch.empty(B, dtype=torch.uint8, device=dev)
         self.h2d_bytes = self.actions_host.numel() * 4
-        self.d2h_bytes = self.obs_host.numel() * 4 + B * 4 + 2 * B
+        self.d2h_bytes = self.obs_host.numel() * self.obs_host.element_size() + B * 4 + 2 * B
         # the pipeline's two side streams and events belong to this stepper (marlnav_host_pipe)
         self._pipe = ctypes.c_void_p()
         with torch.cuda.device(dev):
@@ -603,14 +638,17 @@ class HostStepper:
             stream = torch.cuda.current_stream(env.device).cuda_stream
             rs = env._reset_spec(alias=env._alias_pending)
             rs.step_counter = env._next_step_counter(stream)
-            _lib.check(env._lib.marlnav_step_host_f32(
-                self._pipe, ctypes.byref(env._c_params), ctypes.byref(rs),
-                p(env.states), p(env.obstacles), p(env.target), p(env._step_num), p(env._terminates_u8),
-                p(src), p(self.actions_dev), p(self.obs_dev), p(self.rewards_dev),
-                p(self.terminated_dev), p(self.truncated_dev),
-                p(self.obs_host), p(self.rewards_host), p(self.terminated_host), p(self.truncated_host),
-                p(env._stats), ctypes.byref(env._io) if env._io is not None else None,
-                ctypes.c_void_p(stream)), "marlnav_step_host_f32")
+            args = (self._pipe, ctypes.byref(env._c_params), ctypes.byref(rs),
+                    p(env.states), p(env.obstacles), p(env.target), p(env._step_num), p(env._terminates_u8),
+                    p(src), p(self.actions_dev), p(self.obs_dev), p(self.rewards_dev),
+                    p(self.terminated_dev), p(self.truncated_dev),
+                    p(self.obs_host), p(self.rewards_host), p(self.terminated_host), p(self.truncated_host),
+                    p(env._stats), ctypes.byref(env._io) if env._io is not None else None,
+                    ctypes.c_void_p(stream))
+            if env._obs_code == 0:
+                _lib.check(env._lib.marlnav_step_host_f32(*args), "marlnav_step_host_f32")
+            else:
+                _lib.check(env._lib.marlnav_step_host_typed(*args, env._obs_code), "marlnav_step_host_typed")
             env._commit_step_counter()
             if env._alias_pending:
                 env._tmpl_states = env.states.clone()

@@ -209,6 +209,13 @@ def discounted_returns(rewards, done, gamma, normalize=False):
     return out
 
 
+def _require_f32_obs(env, what):
+    """The rollout buffers, the fused actor and the critic read float32 observations."""
+    if env.obs_dtype != torch.float32:
+        raise _lib.MarlnavError(f"{what} needs an env with float32 observations; this env's obs_dtype is "
+                                f"{env.obs_dtype}")
+
+
 @torch.no_grad()
 def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None, scaler_params=None,
                     fuse_actor=True):
@@ -223,7 +230,8 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
 
     ``fuse_actor``: sample the actions inside the step launch (``marlnav_act_step_f32``: one launch
     per iteration instead of two) where that kernel exists -- 3 agents, 1..6 obstacles; same bits
-    either way (``test_fused_actor_step_matches_two_launches``)."""
+    either way (``test_fused_actor_step_matches_two_launches``).  Float32 observations only."""
+    _require_f32_obs(env, "collect_rollout")
     if normalizer_params is not None or scaler_params is not None:
         env.fuse_io(normalizer_params, scaler_params)
     if env._io is None or not env._io.obs_mean or not env._io.act_scale:
@@ -288,6 +296,7 @@ class RolloutGraph:
     ``replay()`` returns the SAME buffer tensors every time (clone what must outlive the next replay)."""
 
     def __init__(self, env, actor, buffer_len, critic=None, warmup_steps=2):
+        _require_f32_obs(env, "RolloutGraph")
         if critic is not None and not isinstance(critic, FusedCritic):
             raise _lib.MarlnavError("RolloutGraph needs a FusedCritic (or no critic)")
         self.env, self.actor, self.critic, self.buffer_len = env, actor, critic, int(buffer_len)
@@ -376,6 +385,7 @@ class MappoRollout:
 
     def __init__(self, mappo, use_graph=True, seed=None):
         env = mappo.env
+        _require_f32_obs(env, "MappoRollout")
         self.mappo, self.env, self.use_graph = mappo, env, bool(use_graph)
         norm, scal = mappo._normalize, mappo._scale_up
         env.fuse_io_tensors(norm.mean, norm.scale_tensor.reshape(-1, env.obs_size)[0],
