@@ -290,7 +290,8 @@ const char* marlnav_rollout_last_error(void);
 }
 #endif
 
-/* float16 / bfloat16 observations: the `_typed` entry points */
+/* float16 / bfloat16 observations: the `_typed` entry points of the step, then of the rollout */
 #include "marlnav_b200_typed.h"
+#include "marlnav_b200_rollout_typed.h"
 
 #endif /* MARLNAV_B200_H */

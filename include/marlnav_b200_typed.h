@@ -14,8 +14,9 @@
  *
  * A 16-bit `obs` may start at any 2-byte aligned address; 16-byte aligned buffers take the bulk
  * (TMA) stores, others plain stores with the same results.  An unknown `obs_dtype` returns
- * MARLNAV_ERR_BAD_ARG before anything is launched.  The fused actor (marlnav_act_step_f32) reads
- * and writes float32 observations only, and marlnav_step_launch_info reports the float32 kernels.
+ * MARLNAV_ERR_BAD_ARG before anything is launched.  marlnav_step_launch_info reports the float32
+ * kernels.  The 16-bit actor, critic and fused actor+step entries are declared in
+ * marlnav_b200_rollout_typed.h.
  */
 #ifndef MARLNAV_B200_TYPED_H
 #define MARLNAV_B200_TYPED_H

@@ -23,6 +23,9 @@ EXPORTS = ("marlnav_abi_version", "marlnav_last_error", "marlnav_obs_size", "mar
            "marlnav_rollout_last_error")
 # every symbol include/marlnav_b200_typed.h declares (16-bit observations; included by marlnav_b200.h)
 TYPED_EXPORTS = ("marlnav_observe_typed", "marlnav_step_typed", "marlnav_step_call_typed", "marlnav_step_host_typed")
+# every symbol include/marlnav_b200_rollout_typed.h declares (16-bit observations into the actor, the
+# critic and the fused actor+step; included by marlnav_b200.h)
+ROLLOUT_TYPED_EXPORTS = ("marlnav_actor_sample_typed", "marlnav_critic_value_typed", "marlnav_act_step_typed")
 
 
 class _Sized(ctypes.Structure):
@@ -107,7 +110,7 @@ def load():
     lib.marlnav_rollout_last_error.restype = ctypes.c_char_p
     sizeofs = ("marlnav_sizeof_env_params", "marlnav_sizeof_reset_spec", "marlnav_sizeof_io_transform",
                "marlnav_sizeof_actor_spec", "marlnav_sizeof_step_call")
-    for name in EXPORTS + TYPED_EXPORTS:
+    for name in EXPORTS + TYPED_EXPORTS + ROLLOUT_TYPED_EXPORTS:
         if name in sizeofs:
             getattr(lib, name).restype = ctypes.c_size_t
         elif name == "marlnav_host_pipe_destroy":
@@ -133,6 +136,9 @@ def load():
     lib.marlnav_counter_add.argtypes = [vp, u64, vp]
     lib.marlnav_discounted_returns_f64.argtypes = [vp, vp, f64, i32, i64, vp, vp]
     lib.marlnav_critic_value_f32.argtypes = [vp, i64, i32, i32] + [vp] * 6
+    lib.marlnav_actor_sample_typed.argtypes = [vp, i32, i64, i32, i32] + [vp] * 7 + [u64, u64, vp, u64] + [vp] * 5
+    lib.marlnav_critic_value_typed.argtypes = [vp, i32, i64, i32, i32] + [vp] * 6
+    lib.marlnav_act_step_typed.argtypes = [vp] * 12 + [i32] + [vp] * 6
     got = lib.marlnav_abi_version()
     if got != ABI_VERSION:
         raise MarlnavError(f"libmarlnav_b200.so ABI {got} != binding ABI {ABI_VERSION}; rebuild")

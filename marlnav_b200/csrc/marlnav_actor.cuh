@@ -12,11 +12,19 @@
 // eps: given (parity tests), or Philox4x32-10 + Box-Muller addressed by (seed; GLOBAL row, counter).
 // Weights in shared memory in torch.nn.Linear layout: w1 (H,S), b1 (H), w_mu/w_std (2,H).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
 
 namespace mna {
+
+// An observation as the policy and the critic read it: float32 as stored, a 16-bit one widened to
+// float32 (exact for half and bfloat16), so a 16-bit input gives the bits of its .float() copy.
+__device__ __forceinline__ float widen(float x) { return x; }
+__device__ __forceinline__ float widen(__half x) { return __half2float(x); }
+__device__ __forceinline__ float widen(__nv_bfloat16 x) { return __bfloat162float(x); }
 
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                uint32_t k0, uint32_t k1) {

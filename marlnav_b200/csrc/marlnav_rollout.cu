@@ -29,9 +29,11 @@ namespace mnr {
 // (models.py:29-31): h = fc1(x); mu = tanh(fc_mu(h)); "std" = softplus(fc_std(h)), and that
 // "std" is used as the diagonal COVARIANCE of MultivariateNormal (models.py:32-34), so the
 // standard deviation of the sampled action is sqrt(softplus(.)).
-template <int MAX_S, int MAX_H>
+//
+// IT: the observations' element type (float, __half, __nv_bfloat16), widened exactly on load.
+template <int MAX_S, int MAX_H, class IT = float>
 __global__ void __launch_bounds__(128)
-actor_sample_kernel(const float* __restrict__ obs, long long N, int S, int H,
+actor_sample_kernel(const IT* __restrict__ obs, long long N, int S, int H,
                     const float* __restrict__ w1, const float* __restrict__ b1,
                     const float* __restrict__ w_mu, const float* __restrict__ b_mu,
                     const float* __restrict__ w_std, const float* __restrict__ b_std,
@@ -47,7 +49,7 @@ actor_sample_kernel(const float* __restrict__ obs, long long N, int S, int H,
 
     float x[MAX_S];
 #pragma unroll
-    for (int k = 0; k < MAX_S; ++k) x[k] = k < S ? obs[row * S + k] : 0.f;
+    for (int k = 0; k < MAX_S; ++k) x[k] = k < S ? mna::widen(obs[row * S + k]) : 0.f;
     if (counter_dev) counter += __ldg(counter_dev);      // host value = offset inside a batch
     const mna::ActorOut o = mna::actor_row<MAX_S>(x, S, H, mna::ActorWeights(sm, S, H), b_mu, b_std, eps, seed, counter, row,
                                                       row_offset + (uint64_t)row);
@@ -58,9 +60,10 @@ actor_sample_kernel(const float* __restrict__ obs, long long N, int S, int H,
 }
 
 // Critic.forward (models.py:39-56): value = fc2(relu(fc1(flatten(x)))), one thread per env.
-template <int MAX_H>
+// IT, in all three critic kernels: the observations' element type, widened exactly on load.
+template <int MAX_H, class IT = float>
 __global__ void __launch_bounds__(128)
-critic_value_kernel(const float* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
+critic_value_kernel(const IT* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
                     const float* __restrict__ b1, const float* __restrict__ w2, const float* __restrict__ b2,
                     float* __restrict__ values) {
     extern __shared__ float sm[];
@@ -72,9 +75,9 @@ critic_value_kernel(const float* __restrict__ obs, long long B, int K, int H, co
     float h[MAX_H];
 #pragma unroll
     for (int j = 0; j < MAX_H; ++j) h[j] = j < H ? b1[j] : 0.f;
-    const float* x = obs + e * K;
+    const IT* x = obs + e * K;
     for (int k = 0; k < K; ++k) {
-        const float xk = x[k];
+        const float xk = mna::widen(x[k]);
 #pragma unroll
         for (int j = 0; j < MAX_H; ++j)
             if (j < H) h[j] = fmaf(xk, s_w1[k * H + j], h[j]);
@@ -90,9 +93,9 @@ critic_value_kernel(const float* __restrict__ obs, long long B, int K, int H, co
 // thread per env is a 1 800-step serial chain on a handful of warps: here 64 lanes share an env, one
 // hidden unit each (K steps), and one lane finishes the H-term output sum.  Same summation orders
 // as critic_value_kernel, hence the same bits.  4 envs in flight per CTA.
-template <int MAX_H>
+template <int MAX_H, class IT = float>
 __global__ void __launch_bounds__(4 * MAX_H)
-critic_value_wide_kernel(const float* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
+critic_value_wide_kernel(const IT* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
                          const float* __restrict__ b1, const float* __restrict__ w2, const float* __restrict__ b2,
                          float* __restrict__ values) {
     extern __shared__ float sm[];
@@ -105,9 +108,9 @@ critic_value_wide_kernel(const float* __restrict__ obs, long long B, int K, int 
     for (long long e0 = (long long)blockIdx.x * 4; e0 < B; e0 += stride) {      // uniform trip count per CTA
         const long long e = e0 + g;
         if (e < B && j < H) {
-            const float* x = obs + e * K;
+            const IT* x = obs + e * K;
             float h = b1[j];
-            for (int k = 0; k < K; ++k) h = fmaf(__ldg(x + k), s_w1[k * H + j], h);
+            for (int k = 0; k < K; ++k) h = fmaf(mna::widen(__ldg(x + k)), s_w1[k * H + j], h);
             s_h[g * MAX_H + j] = fmaxf(h, 0.f);
         }
         __syncthreads();
@@ -123,9 +126,9 @@ critic_value_wide_kernel(const float* __restrict__ obs, long long B, int K, int 
 // Mid-sized batches: L = 16 or 4 lanes per env inside one warp, each lane owning the hidden units
 // j = l, l + L, ... (independent K-step chains), lane 0 of the group finishing the H-term sum.
 // Same summation orders again.
-template <int L, int MAX_H>
+template <int L, int MAX_H, class IT = float>
 __global__ void __launch_bounds__(128)
-critic_value_group_kernel(const float* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
+critic_value_group_kernel(const IT* __restrict__ obs, long long B, int K, int H, const float* __restrict__ w1,
                           const float* __restrict__ b1, const float* __restrict__ w2, const float* __restrict__ b2,
                           float* __restrict__ values) {
     constexpr int PER = (MAX_H + L - 1) / L;             // hidden units per lane
@@ -140,12 +143,12 @@ critic_value_group_kernel(const float* __restrict__ obs, long long B, int K, int
     for (long long e0 = (long long)blockIdx.x * GROUPS; e0 < B; e0 += stride) {     // uniform trip count per CTA
         const long long e = e0 + g;
         if (e < B) {
-            const float* x = obs + e * K;
+            const IT* x = obs + e * K;
             float h[PER];
 #pragma unroll
             for (int u = 0; u < PER; ++u) h[u] = (l + u * L) < H ? b1[l + u * L] : 0.f;
             for (int k = 0; k < K; ++k) {
-                const float xk = __ldg(x + k);
+                const float xk = mna::widen(__ldg(x + k));
 #pragma unroll
                 for (int u = 0; u < PER; ++u)
                     if ((l + u * L) < H) h[u] = fmaf(xk, s_w1[k * H + l + u * L], h[u]);
@@ -197,23 +200,21 @@ __global__ void discounted_returns_kernel(const float* __restrict__ rewards, con
 
 namespace {
 thread_local char g_err2[256] = "";
-}
 
-extern "C" {
-
-const char* marlnav_rollout_last_error(void) { return g_err2; }
-
-int marlnav_actor_sample_f32(const float* obs, long long N, int S, int H, const float* w1, const float* b1,
-                             const float* w_mu, const float* b_mu, const float* w_std, const float* b_std,
-                             const float* eps, uint64_t seed, uint64_t counter, const uint64_t* counter_dev,
-                             uint64_t row_offset,
-                             float* actions, float* log_probs, float* mu_out, float* var_out, void* stream) {
+// The bodies of the `_f32` and `_typed` rollout entries; IT = the observations' element type and
+// `fn` the entry's name for the error message.
+template <class IT>
+int actor_sample(const char* fn, const IT* obs, long long N, int S, int H, const float* w1, const float* b1,
+                 const float* w_mu, const float* b_mu, const float* w_std, const float* b_std,
+                 const float* eps, uint64_t seed, uint64_t counter, const uint64_t* counter_dev,
+                 uint64_t row_offset,
+                 float* actions, float* log_probs, float* mu_out, float* var_out, void* stream) {
     if (!obs || !w1 || !b1 || !w_mu || !b_mu || !w_std || !b_std || !actions || !log_probs || N < 1) {
-        snprintf(g_err2, sizeof g_err2, "marlnav_actor_sample_f32: NULL pointer or empty batch");
+        snprintf(g_err2, sizeof g_err2, "%s: NULL pointer or empty batch", fn);
         return MARLNAV_ERR_BAD_ARG;
     }
     if (S < 1 || S > 64 || H < 1 || H > 256) {
-        snprintf(g_err2, sizeof g_err2, "marlnav_actor_sample_f32: need 1 <= obs_size <= 64 and 1 <= hidden <= 256");
+        snprintf(g_err2, sizeof g_err2, "%s: need 1 <= obs_size <= 64 and 1 <= hidden <= 256", fn);
         return MARLNAV_ERR_BAD_SHAPE;
     }
     const int threads = 128;
@@ -226,21 +227,21 @@ int marlnav_actor_sample_f32(const float* obs, long long N, int S, int H, const 
         int dev0 = 0; cudaGetDevice(&dev0);
         if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
             const int max_smem = (256 * 64 + 5 * 256) * (int)sizeof(float);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
             carve[dev0 & 63].store(true, std::memory_order_release);
         }
     }
     if (S <= 16)
-        mnr::actor_sample_kernel<16, 256><<<(unsigned)grid, threads, smem, st>>>(
+        mnr::actor_sample_kernel<16, 256, IT><<<(unsigned)grid, threads, smem, st>>>(
             obs, N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps, seed, counter,
             reinterpret_cast<const unsigned long long*>(counter_dev), row_offset, actions, log_probs, mu_out, var_out);
     else
-        mnr::actor_sample_kernel<64, 256><<<(unsigned)grid, threads, smem, st>>>(
+        mnr::actor_sample_kernel<64, 256, IT><<<(unsigned)grid, threads, smem, st>>>(
             obs, N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps, seed, counter,
             reinterpret_cast<const unsigned long long*>(counter_dev), row_offset, actions, log_probs, mu_out, var_out);
     cudaError_t e = cudaGetLastError();
@@ -248,14 +249,15 @@ int marlnav_actor_sample_f32(const float* obs, long long N, int S, int H, const 
     return 0;
 }
 
-int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const float* w1, const float* b1,
-                             const float* w2, const float* b2, float* values, void* stream) {
+template <class IT>
+int critic_value(const char* fn, const IT* obs, long long B, int K, int H, const float* w1, const float* b1,
+                 const float* w2, const float* b2, float* values, void* stream) {
     if (!obs || !w1 || !b1 || !w2 || !b2 || !values || B < 1) {
-        snprintf(g_err2, sizeof g_err2, "marlnav_critic_value_f32: NULL pointer or empty batch");
+        snprintf(g_err2, sizeof g_err2, "%s: NULL pointer or empty batch", fn);
         return MARLNAV_ERR_BAD_ARG;
     }
     if (K < 1 || H < 1 || H > 64 || (size_t)H * K * sizeof(float) > 200 * 1024) {
-        snprintf(g_err2, sizeof g_err2, "marlnav_critic_value_f32: need hidden <= 64 and hidden*inputs*4 <= 200 KiB");
+        snprintf(g_err2, sizeof g_err2, "%s: need hidden <= 64 and hidden*inputs*4 <= 200 KiB", fn);
         return MARLNAV_ERR_BAD_SHAPE;
     }
     if (B > 2048 && B <= 262144 && (size_t)(H * K + 32 * 64) * sizeof(float) <= 48 * 1024) {
@@ -263,9 +265,9 @@ int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const 
         static std::atomic<bool> carve[64];
         int dev0 = 0; cudaGetDevice(&dev0);
         if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
-            cudaFuncSetAttribute(mnr::critic_value_group_kernel<16, 64>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(mnr::critic_value_group_kernel<16, 64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::critic_value_group_kernel<4, 64>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(mnr::critic_value_group_kernel<4, 64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
             carve[dev0 & 63].store(true, std::memory_order_release);
         }
@@ -277,9 +279,9 @@ int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const 
         const unsigned grid = (unsigned)(want < cap ? want : cap);
         const size_t smem = (size_t)(H * K + groups * 64) * sizeof(float);
         if (l16)
-            mnr::critic_value_group_kernel<16, 64><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
+            mnr::critic_value_group_kernel<16, 64, IT><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
         else
-            mnr::critic_value_group_kernel<4, 64><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
+            mnr::critic_value_group_kernel<4, 64, IT><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value_group launch: %s", cudaGetErrorString(e)); return (int)e; }
         return 0;
@@ -293,11 +295,11 @@ int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const 
         static std::atomic<bool> carve[64];
         int dev0 = 0; cudaGetDevice(&dev0);
         if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
-            cudaFuncSetAttribute(mnr::critic_value_wide_kernel<64>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(mnr::critic_value_wide_kernel<64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
             carve[dev0 & 63].store(true, std::memory_order_release);
         }
-        mnr::critic_value_wide_kernel<64><<<grid, 256, (size_t)(H * K + 4 * 64) * sizeof(float), (cudaStream_t)stream>>>(
+        mnr::critic_value_wide_kernel<64, IT><<<grid, 256, (size_t)(H * K + 4 * 64) * sizeof(float), (cudaStream_t)stream>>>(
             obs, B, K, H, w1, b1, w2, b2, values);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value_wide launch: %s", cudaGetErrorString(e)); return (int)e; }
@@ -308,14 +310,75 @@ int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const 
     static std::atomic<bool> big_smem[64];
     int dev = 0; cudaGetDevice(&dev);
     if (smem > 48 * 1024 && !big_smem[dev & 63].load(std::memory_order_acquire)) {
-        cudaFuncSetAttribute(mnr::critic_value_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaFuncSetAttribute(mnr::critic_value_kernel<64, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         big_smem[dev & 63].store(true, std::memory_order_release);
     }
-    mnr::critic_value_kernel<64><<<(unsigned)((B + threads - 1) / threads), threads, smem, (cudaStream_t)stream>>>(
+    mnr::critic_value_kernel<64, IT><<<(unsigned)((B + threads - 1) / threads), threads, smem, (cudaStream_t)stream>>>(
         obs, B, K, H, w1, b1, w2, b2, values);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value launch: %s", cudaGetErrorString(e)); return (int)e; }
     return 0;
+}
+
+bool obs_dtype_ok(int obs_dtype) {
+    if (obs_dtype == MARLNAV_OBS_F32 || obs_dtype == MARLNAV_OBS_F16 || obs_dtype == MARLNAV_OBS_BF16) return true;
+    snprintf(g_err2, sizeof g_err2,
+             "obs_dtype must be MARLNAV_OBS_F32 (0), MARLNAV_OBS_F16 (1) or MARLNAV_OBS_BF16 (2), got %d", obs_dtype);
+    return false;
+}
+
+}  // namespace
+
+extern "C" {
+
+const char* marlnav_rollout_last_error(void) { return g_err2; }
+
+int marlnav_actor_sample_f32(const float* obs, long long N, int S, int H, const float* w1, const float* b1,
+                             const float* w_mu, const float* b_mu, const float* w_std, const float* b_std,
+                             const float* eps, uint64_t seed, uint64_t counter, const uint64_t* counter_dev,
+                             uint64_t row_offset,
+                             float* actions, float* log_probs, float* mu_out, float* var_out, void* stream) {
+    return actor_sample("marlnav_actor_sample_f32", obs, N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps, seed,
+                        counter, counter_dev, row_offset, actions, log_probs, mu_out, var_out, stream);
+}
+
+int marlnav_actor_sample_typed(const void* obs, int obs_dtype, long long N, int S, int H, const float* w1,
+                               const float* b1, const float* w_mu, const float* b_mu, const float* w_std,
+                               const float* b_std, const float* eps, uint64_t seed, uint64_t counter,
+                               const uint64_t* counter_dev, uint64_t row_offset,
+                               float* actions, float* log_probs, float* mu_out, float* var_out, void* stream) {
+    if (!obs_dtype_ok(obs_dtype)) return MARLNAV_ERR_BAD_ARG;
+    const char* fn = "marlnav_actor_sample_typed";
+    switch (obs_dtype) {
+        case MARLNAV_OBS_F16:
+            return actor_sample(fn, static_cast<const __half*>(obs), N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps,
+                                seed, counter, counter_dev, row_offset, actions, log_probs, mu_out, var_out, stream);
+        case MARLNAV_OBS_BF16:
+            return actor_sample(fn, static_cast<const __nv_bfloat16*>(obs), N, S, H, w1, b1, w_mu, b_mu, w_std, b_std,
+                                eps, seed, counter, counter_dev, row_offset, actions, log_probs, mu_out, var_out, stream);
+        default:
+            return actor_sample(fn, static_cast<const float*>(obs), N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps,
+                                seed, counter, counter_dev, row_offset, actions, log_probs, mu_out, var_out, stream);
+    }
+}
+
+int marlnav_critic_value_f32(const float* obs, long long B, int K, int H, const float* w1, const float* b1,
+                             const float* w2, const float* b2, float* values, void* stream) {
+    return critic_value("marlnav_critic_value_f32", obs, B, K, H, w1, b1, w2, b2, values, stream);
+}
+
+int marlnav_critic_value_typed(const void* obs, int obs_dtype, long long B, int K, int H, const float* w1,
+                               const float* b1, const float* w2, const float* b2, float* values, void* stream) {
+    if (!obs_dtype_ok(obs_dtype)) return MARLNAV_ERR_BAD_ARG;
+    const char* fn = "marlnav_critic_value_typed";
+    switch (obs_dtype) {
+        case MARLNAV_OBS_F16:
+            return critic_value(fn, static_cast<const __half*>(obs), B, K, H, w1, b1, w2, b2, values, stream);
+        case MARLNAV_OBS_BF16:
+            return critic_value(fn, static_cast<const __nv_bfloat16*>(obs), B, K, H, w1, b1, w2, b2, values, stream);
+        default:
+            return critic_value(fn, static_cast<const float*>(obs), B, K, H, w1, b1, w2, b2, values, stream);
+    }
 }
 
 int marlnav_discounted_returns_f64(const float* rewards, const uint8_t* done, double gamma, int T, long long B,

@@ -302,24 +302,31 @@ class Env(object):
         return self._sampler()
 
     def supports_fused_actor(self, actor):
-        """Is there a fused {actor -> step} kernel for this env and actor (marlnav_act_step_f32)?
-        Not for 16-bit observations: the fused actor reads and writes float32."""
-        return (self.obs_dtype == torch.float32 and self.num_agents == 3 and 1 <= self.num_obstacles <= 6 and self._io is not None
+        """Is there a fused {actor -> step} kernel for this env and actor (marlnav_act_step_f32, or
+        marlnav_act_step_typed for 16-bit observations)?"""
+        return (self.num_agents == 3 and 1 <= self.num_obstacles <= 6 and self._io is not None
                 and bool(self._io.obs_mean) and bool(self._io.act_scale)
                 and getattr(actor, 'obs_size', None) == self.obs_size and getattr(actor, 'hidden', 10 ** 9) <= 256
                 and getattr(getattr(actor, 'w1', None), 'device', None) == self.states.device)
 
-    def act_step_fused(self, actor, obs_in, out):
+    def act_step_fused(self, actor, obs_in, out, obs_dtype=torch.float32):
         """``actor.act(obs_in)`` + ``step_fused`` as ONE launch (SURVEY 8(f)-2; models.py:113-122).
         ``obs_in`` (B,A,S): the normalised observations of the current state; ``out`` = preallocated
         (actions (B*A,2), log_probs (B*A), next_obs (B,A,S), rewards (B), terminated_u8 (B),
-        truncated_u8 (B)).  Needs ``fuse_io`` with both transforms and float32 observations."""
-        if self.obs_dtype != torch.float32:
-            raise _lib.MarlnavError(f"act_step_fused reads and writes float32 observations; this env's obs_dtype "
-                                    f"is {self.obs_dtype}")
+        truncated_u8 (B)).  Needs ``fuse_io`` with both transforms.  ``obs_dtype`` is the element type
+        of ``obs_in`` and ``next_obs`` and must be the env's ``obs_dtype``: the actor reads 16-bit
+        observations widened exactly to float32, the same bits as ``actor.act(obs_in.float())``."""
+        if obs_dtype != self.obs_dtype:
+            raise _lib.MarlnavError(f"act_step_fused: obs_dtype {obs_dtype} does not match this env's obs_dtype "
+                                    f"{self.obs_dtype}")
         if not self.supports_fused_actor(actor):
             raise _lib.MarlnavError("no fused actor+step kernel for this env/actor (see supports_fused_actor)")
         actions, log_probs, obs, rew, term, trunc = out
+        n = self.num_parallel * self.num_agents * self.obs_size
+        for name, t in (("obs_in", obs_in), ("out[2]", obs)):
+            if t.dtype != obs_dtype or t.numel() < n:
+                raise _lib.MarlnavError(f"act_step_fused: {name} must be {obs_dtype} with at least {n} elements, "
+                                        f"got {t.dtype} with {t.numel()}")
         if obs_in.data_ptr() == obs.data_ptr():
             raise _lib.MarlnavError("act_step_fused: obs_in and the output observations must be different buffers")
         with torch.cuda.device(self.device):
@@ -328,12 +335,15 @@ class Env(object):
             sp.row_offset = self._env_id_offset * self.num_agents if actor.row_offset is None else actor.row_offset
             rs = self._reset_spec(alias=self._alias_pending)
             rs.step_counter = self._next_step_counter(stream)
-            _lib.check(self._lib.marlnav_act_step_f32(
-                ctypes.byref(self._c_params), ctypes.byref(rs), self._ptr(self.states), self._ptr(self.obstacles),
-                self._ptr(self.target), self._ptr(self._step_num), self._ptr(self._terminates_u8),
-                ctypes.byref(sp), obs_in.data_ptr(), actions.data_ptr(), log_probs.data_ptr(),
-                obs.data_ptr(), rew.data_ptr(), term.data_ptr(), trunc.data_ptr(), self._ptr(self._stats),
-                ctypes.byref(self._io), stream), "marlnav_act_step_f32")
+            head = (ctypes.byref(self._c_params), ctypes.byref(rs), self._ptr(self.states), self._ptr(self.obstacles),
+                    self._ptr(self.target), self._ptr(self._step_num), self._ptr(self._terminates_u8),
+                    ctypes.byref(sp), obs_in.data_ptr(), actions.data_ptr(), log_probs.data_ptr(), obs.data_ptr())
+            tail = (rew.data_ptr(), term.data_ptr(), trunc.data_ptr(), self._ptr(self._stats),
+                    ctypes.byref(self._io), stream)
+            if self._obs_code == 0:
+                _lib.check(self._lib.marlnav_act_step_f32(*head, *tail), "marlnav_act_step_f32")
+            else:
+                _lib.check(self._lib.marlnav_act_step_typed(*head, self._obs_code, *tail), "marlnav_act_step_typed")
             self._commit_step_counter()
             if self._alias_pending:
                 # the reference's template froze at "state after the first move" (B-6)
@@ -431,19 +441,26 @@ class Env(object):
         self._io, self._io_tensors = (io, keep) if keep else (None, None)
         self.__dict__.pop('_call_cache', None)
 
+    def _observations_f32(self):
+        """(B,A,S) float32 observations of the current states, whatever ``obs_dtype`` is: a 16-bit
+        rollout normalises these before it rounds them (``collect_rollout``)."""
+        with torch.cuda.device(self.device):
+            obs = torch.empty(self.num_parallel, self.num_agents, self.obs_size, device=self.device)
+            _lib.check(self._lib.marlnav_observe_f32(
+                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
+                self._ptr(self.target), self._ptr(obs), self._stream()), "marlnav_observe_f32")
+        return obs
+
     def observations_fused(self):
         """(B,A,S) observation buffer of the current states, in ``obs_dtype`` (one kernel launch)."""
+        if self._obs_code == 0:
+            return self._observations_f32()
         B, A = self.num_parallel, self.num_agents
         with torch.cuda.device(self.device):
             obs = torch.empty(B, A, self.obs_size, dtype=self.obs_dtype, device=self.device)
-            if self._obs_code == 0:
-                _lib.check(self._lib.marlnav_observe_f32(
-                    ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
-                    self._ptr(self.target), self._ptr(obs), self._stream()), "marlnav_observe_f32")
-            else:
-                _lib.check(self._lib.marlnav_observe_typed(
-                    ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
-                    self._ptr(self.target), self._ptr(obs), self._obs_code, self._stream()), "marlnav_observe_typed")
+            _lib.check(self._lib.marlnav_observe_typed(
+                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
+                self._ptr(self.target), self._ptr(obs), self._obs_code, self._stream()), "marlnav_observe_typed")
         return obs
 
     def observations(self):

@@ -2,13 +2,15 @@
 
 * ``FusedActor``          -- the reference's ``Actor.forward`` + ``dist.sample()`` +
                              ``dist.log_prob()`` (/root/reference/marlnav/models.py:27-36,113-115)
-                             as one kernel launch (``marlnav_actor_sample_f32``).
+                             as one kernel launch (``marlnav_actor_sample_f32``, or
+                             ``marlnav_actor_sample_typed`` for float16 / bfloat16 observations).
 * ``discounted_returns``  -- the backward scan of ``MAPPO._process_rewards``
                              (models.py:131-139) as one kernel (``marlnav_discounted_returns_f64``),
                              optionally followed by its std/mean normalisation (models.py:141-145).
 * ``collect_rollout``     -- ``MAPPO.get_data`` (models.py:106-129) with device-resident (T, ...)
                              buffers instead of a Python list of lists: per step one actor launch and
-                             one fused environment step (normaliser and action scaler folded in).
+                             one fused environment step (normaliser and action scaler folded in); the
+                             observation buffer in the env's ``obs_dtype`` when the caller opts in.
 
 The reference's learner itself (PPO losses, Adam) is out of scope and stays stock PyTorch; these
 functions hand it tensors in the layouts it already uses.
@@ -18,6 +20,7 @@ import ctypes
 import torch
 
 from . import _lib
+from .env import OBS_DTYPES
 
 
 def _rollout_check(rc, what):
@@ -113,12 +116,16 @@ class FusedActor:
         buffer).  Returns ``(actions (N,2), log_probs (N,))`` with N = prod(leading dims), exactly
         what models.py:113-115 produces; ``eps`` (N,2) injects the normal draws (tests); ``out`` =
         preallocated contiguous ``(actions, log_probs)`` tensors to write into; ``row_offset``
-        overrides ``self.row_offset`` for this call."""
+        overrides ``self.row_offset`` for this call.  float16 / bfloat16 ``obs`` are read as they
+        are and widened exactly in the kernel: the same bits as ``act(obs.float())``.  Other dtypes
+        are converted to float32 first.  The outputs are float32."""
         if row_offset is None:
             row_offset = self.row_offset or 0
         x = obs.reshape(-1, self.obs_size)
-        if x.dtype != torch.float32 or not x.is_contiguous() or x.device != self.device:
-            x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        code = OBS_DTYPES.get(x.dtype, 0)
+        dtype = x.dtype if code else torch.float32
+        if x.dtype != dtype or not x.is_contiguous() or x.device != self.device:
+            x = x.to(device=self.device, dtype=dtype).contiguous()
         n = x.shape[0]
         with torch.cuda.device(self.device):
             if out is not None:
@@ -133,10 +140,13 @@ class FusedActor:
             p = lambda t: t.data_ptr() if t is not None else None
             stream = torch.cuda.current_stream(self.device).cuda_stream
             counter = self._advance_counter(stream)
-            _rollout_check(self._lib.marlnav_actor_sample_f32(
-                p(x), n, self.obs_size, self.hidden, p(self.w1), p(self.b1), p(self.w_mu), p(self.b_mu),
-                p(self.w_std), p(self.b_std), p(eps), self.seed, counter, p(self._counter_dev), int(row_offset),
-                p(actions), p(log_probs), p(mu), p(var), stream), "marlnav_actor_sample_f32")
+            args = (n, self.obs_size, self.hidden, p(self.w1), p(self.b1), p(self.w_mu), p(self.b_mu),
+                    p(self.w_std), p(self.b_std), p(eps), self.seed, counter, p(self._counter_dev), int(row_offset),
+                    p(actions), p(log_probs), p(mu), p(var), stream)
+            if code == 0:
+                _rollout_check(self._lib.marlnav_actor_sample_f32(p(x), *args), "marlnav_actor_sample_f32")
+            else:
+                _rollout_check(self._lib.marlnav_actor_sample_typed(p(x), code, *args), "marlnav_actor_sample_typed")
         return (actions, log_probs, mu, var) if want_moments else (actions, log_probs)
 
 
@@ -163,18 +173,26 @@ class FusedCritic:
         self.hidden, self.inputs = self.w1.shape
 
     def __call__(self, obs, out=None):
-        """``obs``: (B, ...) normalised observations with prod(...) == inputs.  Returns (B,1)."""
+        """``obs``: (B, ...) normalised observations with prod(...) == inputs.  Returns (B,1) float32.
+        float16 / bfloat16 ``obs`` are read as they are and widened exactly in the kernel: the same
+        bits as ``self(obs.float())``.  Other dtypes are converted to float32 first."""
         x = obs.reshape(obs.shape[0], -1)
         if x.shape[1] != self.inputs:
             raise _lib.MarlnavError(f"critic expects {self.inputs} inputs per env, got {x.shape[1]}")
-        if x.dtype != torch.float32 or not x.is_contiguous() or x.device != self.device:
-            x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        code = OBS_DTYPES.get(x.dtype, 0)
+        dtype = x.dtype if code else torch.float32
+        if x.dtype != dtype or not x.is_contiguous() or x.device != self.device:
+            x = x.to(device=self.device, dtype=dtype).contiguous()
         with torch.cuda.device(self.device):
             v = out if out is not None else torch.empty(x.shape[0], 1, device=self.device)
-            _rollout_check(self._lib.marlnav_critic_value_f32(
-                x.data_ptr(), x.shape[0], self.inputs, self.hidden, self.w1.data_ptr(), self.b1.data_ptr(),
-                self.w2.data_ptr(), self.b2.data_ptr(), v.data_ptr(),
-                torch.cuda.current_stream(self.device).cuda_stream), "marlnav_critic_value_f32")
+            args = (x.shape[0], self.inputs, self.hidden, self.w1.data_ptr(), self.b1.data_ptr(),
+                    self.w2.data_ptr(), self.b2.data_ptr(), v.data_ptr(),
+                    torch.cuda.current_stream(self.device).cuda_stream)
+            if code == 0:
+                _rollout_check(self._lib.marlnav_critic_value_f32(x.data_ptr(), *args), "marlnav_critic_value_f32")
+            else:
+                _rollout_check(self._lib.marlnav_critic_value_typed(x.data_ptr(), code, *args),
+                               "marlnav_critic_value_typed")
         return v
 
 
@@ -209,8 +227,17 @@ def discounted_returns(rewards, done, gamma, normalize=False):
     return out
 
 
+def _require_obs_dtype(env, obs_dtype, what):
+    """A rollout's observation buffer has the type the caller asked for, and it must be the env's: a
+    16-bit buffer goes to a learner, whose float32 layers refuse it unless it casts, so a 16-bit env
+    never hands one out unasked."""
+    if obs_dtype != env.obs_dtype:
+        raise _lib.MarlnavError(f"{what}: obs_dtype {obs_dtype} does not match the env's obs_dtype {env.obs_dtype} "
+                                f"(pass obs_dtype={env.obs_dtype} for a buffer of that type)")
+
+
 def _require_f32_obs(env, what):
-    """The rollout buffers, the fused actor and the critic read float32 observations."""
+    """MappoRollout hands its buffer to the reference's float32 learner."""
     if env.obs_dtype != torch.float32:
         raise _lib.MarlnavError(f"{what} needs an env with float32 observations; this env's obs_dtype is "
                                 f"{env.obs_dtype}")
@@ -218,7 +245,7 @@ def _require_f32_obs(env, what):
 
 @torch.no_grad()
 def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None, scaler_params=None,
-                    fuse_actor=True):
+                    fuse_actor=True, obs_dtype=torch.float32):
     """``MAPPO.get_data`` (models.py:106-129) on device-resident buffers.
 
     ``env``: a ``marlnav_b200.Env``; ``actor``: a ``FusedActor``; ``critic``: optional ``FusedCritic``
@@ -230,8 +257,14 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
 
     ``fuse_actor``: sample the actions inside the step launch (``marlnav_act_step_f32``: one launch
     per iteration instead of two) where that kernel exists -- 3 agents, 1..6 obstacles; same bits
-    either way (``test_fused_actor_step_matches_two_launches``).  Float32 observations only."""
-    _require_f32_obs(env, "collect_rollout")
+    either way (``test_fused_actor_step_matches_two_launches``).
+
+    ``obs_dtype``: the element type of ``obs`` and ``last_obs``; it must equal ``env.obs_dtype``.
+    With ``torch.float16`` / ``torch.bfloat16`` every stored observation is the normalised float32
+    value rounded to nearest-even (``obs32.to(obs_dtype)``), and the actor and a ``FusedCritic`` read
+    those values widened exactly to float32; a torch-module critic gets ``obs.float()``.  Every other
+    buffer stays float32 (``done``: bool).  Cast learner minibatches with ``.float()``."""
+    _require_obs_dtype(env, obs_dtype, "collect_rollout")
     if normalizer_params is not None or scaler_params is not None:
         env.fuse_io(normalizer_params, scaler_params)
     if env._io is None or not env._io.obs_mean or not env._io.act_scale:
@@ -241,14 +274,15 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
     mean, scale = env._io_tensors[0], env._io_tensors[1]
     # every kernel writes straight into its slice of the buffers: one launch per step on the main
     # stream (two where there is no fused actor kernel), the critic beside it
-    obs_all = torch.empty(T + 1, B, A, S, device=dev)
+    obs_all = torch.empty(T + 1, B, A, S, dtype=obs_dtype, device=dev)
     term = torch.empty(T, B, dtype=torch.uint8, device=dev)
     trunc = torch.empty(T, B, dtype=torch.uint8, device=dev)
     buf = dict(actions=torch.empty(T, B * A, 2, device=dev), log_probs=torch.empty(T, B * A, device=dev),
                rewards=torch.empty(T, B, device=dev))
     if critic is not None:
         buf['values'] = torch.empty(T, B, 1, device=dev)
-    torch.div(env.observations_fused() - mean, scale, out=obs_all[0])          # models.py:110
+    # models.py:110; a 16-bit buffer receives the float32 quotient rounded to nearest-even
+    torch.div(env._observations_f32() - mean, scale, out=obs_all[0])
     # device-resident counters: each step passes its offset, ONE add per counter after the loop
     env.batch_device_counter(True)
     actor.batch_device_counter(True)
@@ -267,11 +301,11 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
                 with torch.cuda.stream(side):
                     critic(obs.view(B, A * S), out=buf['values'][t])            # models.py:120
             if critic is not None and side is None:
-                buf['values'][t].copy_(critic(obs.view(B, A * S)))
+                buf['values'][t].copy_(critic(obs.view(B, A * S).float()))
             if fused:
                 # models.py:113-118,122 in one launch: sample from obs, scale, step, normalise
                 env.act_step_fused(actor, obs, out=(buf['actions'][t], buf['log_probs'][t], obs_all[t + 1],
-                                                    buf['rewards'][t], term[t], trunc[t]))
+                                                    buf['rewards'][t], term[t], trunc[t]), obs_dtype=obs_dtype)
                 continue
             actions, _ = actor.act(obs, out=(buf['actions'][t], buf['log_probs'][t]),     # models.py:113-115
                                    row_offset=actor.row_offset if actor.row_offset is not None else env._env_id_offset * A)
@@ -293,10 +327,11 @@ class RolloutGraph:
     ``buffer_len`` steps becomes one graph launch.  The environment's reset counter and the actor's
     sampling counter live in device memory, so every replay continues the same random streams an
     eager loop would use; ``FusedActor.refresh`` / ``FusedCritic.refresh`` update weights in place.
-    ``replay()`` returns the SAME buffer tensors every time (clone what must outlive the next replay)."""
+    ``replay()`` returns the SAME buffer tensors every time (clone what must outlive the next replay).
+    ``obs_dtype``: the observation buffer's element type, as in ``collect_rollout``."""
 
-    def __init__(self, env, actor, buffer_len, critic=None, warmup_steps=2):
-        _require_f32_obs(env, "RolloutGraph")
+    def __init__(self, env, actor, buffer_len, critic=None, warmup_steps=2, obs_dtype=torch.float32):
+        _require_obs_dtype(env, obs_dtype, "RolloutGraph")
         if critic is not None and not isinstance(critic, FusedCritic):
             raise _lib.MarlnavError("RolloutGraph needs a FusedCritic (or no critic)")
         self.env, self.actor, self.critic, self.buffer_len = env, actor, critic, int(buffer_len)
@@ -307,11 +342,11 @@ class RolloutGraph:
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
             if warmup_steps:                                  # lazy kernel attributes, allocator warm-up
-                collect_rollout(env, actor, warmup_steps, critic=critic)
+                collect_rollout(env, actor, warmup_steps, critic=critic, obs_dtype=obs_dtype)
             side.synchronize()
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph, stream=side):
-                self.buffers = collect_rollout(env, actor, self.buffer_len, critic=critic)
+                self.buffers = collect_rollout(env, actor, self.buffer_len, critic=critic, obs_dtype=obs_dtype)
         torch.cuda.current_stream(dev).wait_stream(side)
 
     def replay(self):
@@ -381,7 +416,10 @@ class MappoRollout:
     views of the rollout's (T, ...) device buffers, valid until the next ``get_data()``.
 
     Differences from the reference's loop: the exploration noise is an addressed Philox stream
-    instead of torch's global generator (same distribution), and nothing is printed per step."""
+    instead of torch's global generator (same distribution), and nothing is printed per step.
+
+    The env must have float32 observations: the buffer goes straight to the reference's own
+    ``train_actor`` / ``train_critic``, whose float32 layers do not take 16-bit input."""
 
     def __init__(self, mappo, use_graph=True, seed=None):
         env = mappo.env
