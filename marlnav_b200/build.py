@@ -14,6 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(_HERE, "csrc", "marlnav_kernels.cu")
 SRC2 = os.path.join(_HERE, "csrc", "marlnav_rollout.cu")
 DEPS = [SRC, SRC2, os.path.join(_HERE, "csrc", "marlnav_math.cuh"), os.path.join(_HERE, "csrc", "marlnav_actor.cuh"),
+        os.path.join(_HERE, "csrc", "marlnav_launch.cuh"),
         os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200.h"),
         os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_typed.h"),
         os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_rollout_typed.h")]
@@ -35,8 +36,7 @@ def build(force=False, verbose=False):
     """Compile when the library is missing or older than its sources; returns its path."""
     if not force and os.path.exists(LIB) and all(os.path.getmtime(LIB) >= os.path.getmtime(d) for d in DEPS):
         return LIB
-    extra = os.environ.get("MARLNAV_NVCC_EXTRA", "").split()      # extra -D flags for A/B builds
-    cmd = [nvcc_path()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB, SRC, SRC2]
+    cmd = [nvcc_path()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB, SRC, SRC2]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or res.returncode != 0:
         sys.stderr.write(res.stdout + res.stderr)

@@ -12,16 +12,12 @@
 // per-row Cholesky of MultivariateNormal around it, and the 1000-iteration Python loop after it.
 #include <cuda_runtime.h>
 #include <math.h>
-#include <atomic>
 #include <stdint.h>
 #include <stdio.h>
 
 #include "../../include/marlnav_b200.h"
 #include "marlnav_actor.cuh"
-
-#ifndef MARLNAV_CRITIC_GROUP_CTAS_PER_SM
-#define MARLNAV_CRITIC_GROUP_CTAS_PER_SM 4
-#endif
+#include "marlnav_launch.cuh"
 
 namespace mnr {
 
@@ -201,6 +197,15 @@ __global__ void discounted_returns_kernel(const float* __restrict__ rewards, con
 namespace {
 thread_local char g_err2[256] = "";
 
+int cuda_fail(cudaError_t e, const char* where) {
+    snprintf(g_err2, sizeof g_err2, "%s: %s", where, cudaGetErrorString(e));
+    return (int)e;
+}
+
+// critic_value_group_kernel: few enough CTAs per SM that the per-CTA weight staging amortises
+// over several env groups
+constexpr int kCriticGroupCtasPerSm = 4;
+
 // The bodies of the `_f32` and `_typed` rollout entries; IT = the observations' element type and
 // `fn` the entry's name for the error message.
 template <class IT>
@@ -221,21 +226,12 @@ int actor_sample(const char* fn, const IT* obs, long long N, int S, int H, const
     const long long grid = (N + threads - 1) / threads;
     const size_t smem = (size_t)(H * S + H + 4 * H) * sizeof(float);
     cudaStream_t st = (cudaStream_t)stream;
-    {   // same shared-memory carveout as the step kernels it alternates with (no SM reconfiguration),
-        // and room for the largest advertised shape (S = 64, H = 256: 69 KiB of weights)
-        static std::atomic<bool> carve[64];
-        int dev0 = 0; cudaGetDevice(&dev0);
-        if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
-            const int max_smem = (256 * 64 + 5 * 256) * (int)sizeof(float);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<16, 256, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-            cudaFuncSetAttribute(mnr::actor_sample_kernel<64, 256, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-            carve[dev0 & 63].store(true, std::memory_order_release);
-        }
-    }
+    // same shared-memory carveout as the step kernels it alternates with, and room for the largest
+    // advertised shape (S = 64, H = 256: 69 KiB of weights)
+    const size_t max_smem = (256 * 64 + 5 * 256) * sizeof(float);
+    cudaError_t e = S <= 16 ? mnl::set_attributes_once<mnr::actor_sample_kernel<16, 256, IT>>(max_smem, true)
+                            : mnl::set_attributes_once<mnr::actor_sample_kernel<64, 256, IT>>(max_smem, true);
+    if (e != cudaSuccess) return cuda_fail(e, "actor_sample attributes");
     if (S <= 16)
         mnr::actor_sample_kernel<16, 256, IT><<<(unsigned)grid, threads, smem, st>>>(
             obs, N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps, seed, counter,
@@ -244,9 +240,8 @@ int actor_sample(const char* fn, const IT* obs, long long N, int S, int H, const
         mnr::actor_sample_kernel<64, 256, IT><<<(unsigned)grid, threads, smem, st>>>(
             obs, N, S, H, w1, b1, w_mu, b_mu, w_std, b_std, eps, seed, counter,
             reinterpret_cast<const unsigned long long*>(counter_dev), row_offset, actions, log_probs, mu_out, var_out);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "actor_sample launch: %s", cudaGetErrorString(e)); return (int)e; }
-    return 0;
+    e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : cuda_fail(e, "actor_sample launch");
 }
 
 template <class IT>
@@ -262,29 +257,21 @@ int critic_value(const char* fn, const IT* obs, long long B, int K, int H, const
     }
     if (B > 2048 && B <= 262144 && (size_t)(H * K + 32 * 64) * sizeof(float) <= 48 * 1024) {
         // mid-sized batches: 16 or 4 lanes per env (see critic_value_group_kernel)
-        static std::atomic<bool> carve[64];
-        int dev0 = 0; cudaGetDevice(&dev0);
-        if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
-            cudaFuncSetAttribute(mnr::critic_value_group_kernel<16, 64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(mnr::critic_value_group_kernel<4, 64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-            carve[dev0 & 63].store(true, std::memory_order_release);
-        }
         const bool l16 = B <= 32768;
+        cudaError_t e = l16 ? mnl::set_attributes_once<mnr::critic_value_group_kernel<16, 64, IT>>(0, true)
+                            : mnl::set_attributes_once<mnr::critic_value_group_kernel<4, 64, IT>>(0, true);
+        if (e != cudaSuccess) return cuda_fail(e, "critic_value_group attributes");
         const int groups = l16 ? 8 : 32;
         const long long want = (B + groups - 1) / groups;
-        // few enough CTAs that the per-CTA weight staging amortises over several env groups
-        const long long cap = 148 * MARLNAV_CRITIC_GROUP_CTAS_PER_SM;
+        const long long cap = 148 * kCriticGroupCtasPerSm;
         const unsigned grid = (unsigned)(want < cap ? want : cap);
         const size_t smem = (size_t)(H * K + groups * 64) * sizeof(float);
         if (l16)
             mnr::critic_value_group_kernel<16, 64, IT><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
         else
             mnr::critic_value_group_kernel<4, 64, IT><<<grid, 128, smem, (cudaStream_t)stream>>>(obs, B, K, H, w1, b1, w2, b2, values);
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value_group launch: %s", cudaGetErrorString(e)); return (int)e; }
-        return 0;
+        e = cudaGetLastError();
+        return e == cudaSuccess ? 0 : cuda_fail(e, "critic_value_group launch");
     }
     if (B <= 2048 && (size_t)(H * K + 4 * 64) * sizeof(float) <= 48 * 1024) {
         // rollout-sized batches: 64 lanes per env (see critic_value_wide_kernel)
@@ -292,32 +279,23 @@ int critic_value(const char* fn, const IT* obs, long long B, int K, int H, const
         const unsigned grid = (unsigned)(want < 148 * 8 ? want : 148 * 8);
         // same shared-memory carveout as the step kernels: SMs need not drain and reconfigure when
         // this runs beside them on a forked stream (collect_rollout)
-        static std::atomic<bool> carve[64];
-        int dev0 = 0; cudaGetDevice(&dev0);
-        if (!carve[dev0 & 63].load(std::memory_order_acquire)) {
-            cudaFuncSetAttribute(mnr::critic_value_wide_kernel<64, IT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-            carve[dev0 & 63].store(true, std::memory_order_release);
-        }
+        cudaError_t e = mnl::set_attributes_once<mnr::critic_value_wide_kernel<64, IT>>(0, true);
+        if (e != cudaSuccess) return cuda_fail(e, "critic_value_wide attributes");
         mnr::critic_value_wide_kernel<64, IT><<<grid, 256, (size_t)(H * K + 4 * 64) * sizeof(float), (cudaStream_t)stream>>>(
             obs, B, K, H, w1, b1, w2, b2, values);
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value_wide launch: %s", cudaGetErrorString(e)); return (int)e; }
-        return 0;
+        e = cudaGetLastError();
+        return e == cudaSuccess ? 0 : cuda_fail(e, "critic_value_wide launch");
     }
     const int threads = 128;
     const size_t smem = (size_t)H * K * sizeof(float);
-    static std::atomic<bool> big_smem[64];
-    int dev = 0; cudaGetDevice(&dev);
-    if (smem > 48 * 1024 && !big_smem[dev & 63].load(std::memory_order_acquire)) {
-        cudaFuncSetAttribute(mnr::critic_value_kernel<64, IT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        big_smem[dev & 63].store(true, std::memory_order_release);
+    if (smem > 48 * 1024) {
+        if (cudaError_t e = mnl::set_attributes_once<mnr::critic_value_kernel<64, IT>>(200 * 1024, false))
+            return cuda_fail(e, "critic_value attributes");
     }
     mnr::critic_value_kernel<64, IT><<<(unsigned)((B + threads - 1) / threads), threads, smem, (cudaStream_t)stream>>>(
         obs, B, K, H, w1, b1, w2, b2, values);
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "critic_value launch: %s", cudaGetErrorString(e)); return (int)e; }
-    return 0;
+    return e == cudaSuccess ? 0 : cuda_fail(e, "critic_value launch");
 }
 
 bool obs_dtype_ok(int obs_dtype) {
@@ -391,8 +369,7 @@ int marlnav_discounted_returns_f64(const float* rewards, const uint8_t* done, do
     mnr::discounted_returns_kernel<<<(unsigned)((B + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
         rewards, done, gamma, T, B, out);
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { snprintf(g_err2, sizeof g_err2, "discounted_returns launch: %s", cudaGetErrorString(e)); return (int)e; }
-    return 0;
+    return e == cudaSuccess ? 0 : cuda_fail(e, "discounted_returns launch");
 }
 
 }  // extern "C"

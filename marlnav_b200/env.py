@@ -302,8 +302,7 @@ class Env(object):
         return self._sampler()
 
     def supports_fused_actor(self, actor):
-        """Is there a fused {actor -> step} kernel for this env and actor (marlnav_act_step_f32, or
-        marlnav_act_step_typed for 16-bit observations)?"""
+        """Is there a fused {actor -> step} kernel (marlnav_act_step_typed) for this env and actor?"""
         return (self.num_agents == 3 and 1 <= self.num_obstacles <= 6 and self._io is not None
                 and bool(self._io.obs_mean) and bool(self._io.act_scale)
                 and getattr(actor, 'obs_size', None) == self.obs_size and getattr(actor, 'hidden', 10 ** 9) <= 256
@@ -335,26 +334,18 @@ class Env(object):
             sp.row_offset = self._env_id_offset * self.num_agents if actor.row_offset is None else actor.row_offset
             rs = self._reset_spec(alias=self._alias_pending)
             rs.step_counter = self._next_step_counter(stream)
-            head = (ctypes.byref(self._c_params), ctypes.byref(rs), self._ptr(self.states), self._ptr(self.obstacles),
-                    self._ptr(self.target), self._ptr(self._step_num), self._ptr(self._terminates_u8),
-                    ctypes.byref(sp), obs_in.data_ptr(), actions.data_ptr(), log_probs.data_ptr(), obs.data_ptr())
-            tail = (rew.data_ptr(), term.data_ptr(), trunc.data_ptr(), self._ptr(self._stats),
-                    ctypes.byref(self._io), stream)
-            if self._obs_code == 0:
-                _lib.check(self._lib.marlnav_act_step_f32(*head, *tail), "marlnav_act_step_f32")
-            else:
-                _lib.check(self._lib.marlnav_act_step_typed(*head, self._obs_code, *tail), "marlnav_act_step_typed")
-            self._commit_step_counter()
-            if self._alias_pending:
-                # the reference's template froze at "state after the first move" (B-6)
-                self._tmpl_states = self.states.clone()
-                self._alias_pending = False
-                self.__dict__.pop('_call_cache', None)      # template pointer changed
+            _lib.check(self._lib.marlnav_act_step_typed(
+                ctypes.byref(self._c_params), ctypes.byref(rs), self._ptr(self.states), self._ptr(self.obstacles),
+                self._ptr(self.target), self._ptr(self._step_num), self._ptr(self._terminates_u8),
+                ctypes.byref(sp), obs_in.data_ptr(), actions.data_ptr(), log_probs.data_ptr(), obs.data_ptr(),
+                self._obs_code, rew.data_ptr(), term.data_ptr(), trunc.data_ptr(), self._ptr(self._stats),
+                ctypes.byref(self._io), stream), "marlnav_act_step_typed")
+            self._step_launched()
         return actions, log_probs, obs, rew, term, trunc
 
     def _next_step_counter(self, stream):
         """``step_counter`` argument of the step about to be launched; nothing on the host moves until
-        ``_commit_step_counter`` is called after the launch was accepted.  Host counter: its next value.
+        ``_step_launched`` is called after the launch was accepted.  Host counter: its next value.
         Device counter: 0 after bumping the device word on ``stream``, or, in batch mode, the step's
         offset inside the batch (``flush_device_counter`` adds the total)."""
         if self._counter_dev is None:
@@ -364,10 +355,17 @@ class Env(object):
         self._lib.marlnav_counter_add(self._counter_dev.data_ptr(), 1, stream)
         return 0
 
-    def _commit_step_counter(self):
+    def _step_launched(self):
+        """Host bookkeeping after a step launch was accepted: the reset step counter moves on, and
+        the first step of an aliased template hands over its template."""
         self._reset_counter += 1
         if self._counter_dev is not None and self._counter_batch:
             self._counter_pending += 1
+        if self._alias_pending:
+            # the reference's template froze at "state after the first move" (B-6)
+            self._tmpl_states = self._states.clone()
+            self._alias_pending = False
+            self.__dict__.pop('_call_cache', None)      # template pointer changed
 
     def batch_device_counter(self, enable=True):
         """Batch mode of the device-resident counter: steps address their Philox draws as
@@ -441,27 +439,23 @@ class Env(object):
         self._io, self._io_tensors = (io, keep) if keep else (None, None)
         self.__dict__.pop('_call_cache', None)
 
+    def _observe(self, dtype):
+        """(B,A,S) observations of the current states in `dtype` (one kernel launch)."""
+        with torch.cuda.device(self.device):
+            obs = torch.empty(self.num_parallel, self.num_agents, self.obs_size, dtype=dtype, device=self.device)
+            _lib.check(self._lib.marlnav_observe_typed(
+                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
+                self._ptr(self.target), self._ptr(obs), OBS_DTYPES[dtype], self._stream()), "marlnav_observe_typed")
+        return obs
+
     def _observations_f32(self):
         """(B,A,S) float32 observations of the current states, whatever ``obs_dtype`` is: a 16-bit
         rollout normalises these before it rounds them (``collect_rollout``)."""
-        with torch.cuda.device(self.device):
-            obs = torch.empty(self.num_parallel, self.num_agents, self.obs_size, device=self.device)
-            _lib.check(self._lib.marlnav_observe_f32(
-                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
-                self._ptr(self.target), self._ptr(obs), self._stream()), "marlnav_observe_f32")
-        return obs
+        return self._observe(torch.float32)
 
     def observations_fused(self):
         """(B,A,S) observation buffer of the current states, in ``obs_dtype`` (one kernel launch)."""
-        if self._obs_code == 0:
-            return self._observations_f32()
-        B, A = self.num_parallel, self.num_agents
-        with torch.cuda.device(self.device):
-            obs = torch.empty(B, A, self.obs_size, dtype=self.obs_dtype, device=self.device)
-            _lib.check(self._lib.marlnav_observe_typed(
-                ctypes.byref(self._c_params), self._ptr(self.states), self._ptr(self.obstacles),
-                self._ptr(self.target), self._ptr(obs), self._obs_code, self._stream()), "marlnav_observe_typed")
-        return obs
+        return self._observe(self.obs_dtype)
 
     def observations(self):
         """environment.py:139-180"""
@@ -509,12 +503,7 @@ class Env(object):
         if c is None:
             rs = self._reset_spec(alias=False)
             self._call_epoch = self.__dict__.get('_call_epoch', 0) + 1
-            if self._obs_code == 0:
-                fn = self._lib.marlnav_step_call_f32
-            else:
-                typed, code = self._lib.marlnav_step_call_typed, self._obs_code
-                fn = lambda call: typed(call, code)
-            c = dict(rs=rs, epoch=self._call_epoch, fn=fn)
+            c = dict(rs=rs, epoch=self._call_epoch)
             self._call_cache = c
         return c
 
@@ -561,15 +550,10 @@ class Env(object):
             rs.alias_first_step = 1
         call.actions = actions.data_ptr()
         call.stream = stream
-        rc = c['fn'](ctypes.addressof(call))
+        rc = self._lib.marlnav_step_call_typed(ctypes.addressof(call), self._obs_code)
         if rc:
-            _lib.check(rc, "marlnav_step_call_f32" if self._obs_code == 0 else "marlnav_step_call_typed")
-        self._commit_step_counter()
-        if self._alias_pending:
-            # the reference's template froze at "state after the first move" (B-6)
-            self._tmpl_states = self._states.clone()
-            self._alias_pending = False
-            self.__dict__.pop('_call_cache', None)      # template pointer changed
+            _lib.check(rc, "marlnav_step_call_typed")
+        self._step_launched()
 
     def step_fused(self, actions, out=None):
         """One fused step.  Returns ``(obs (B,A,S), rewards (B), terminated (B) bool,
@@ -605,7 +589,7 @@ class Env(object):
 
 
 class HostStepper:
-    """Steps an ``Env`` for a HOST-resident policy through ``marlnav_step_host_f32``:
+    """Steps an ``Env`` for a HOST-resident policy through ``marlnav_step_host_typed``:
     pinned host actions in, pinned host observations/rewards/flags out, env state
     resident in HBM.  This is the end-to-end path ``bench.py`` reports as ``e2e``."""
 
@@ -661,15 +645,8 @@ class HostStepper:
                     p(self.terminated_dev), p(self.truncated_dev),
                     p(self.obs_host), p(self.rewards_host), p(self.terminated_host), p(self.truncated_host),
                     p(env._stats), ctypes.byref(env._io) if env._io is not None else None,
-                    ctypes.c_void_p(stream))
-            if env._obs_code == 0:
-                _lib.check(env._lib.marlnav_step_host_f32(*args), "marlnav_step_host_f32")
-            else:
-                _lib.check(env._lib.marlnav_step_host_typed(*args, env._obs_code), "marlnav_step_host_typed")
-            env._commit_step_counter()
-            if env._alias_pending:
-                env._tmpl_states = env.states.clone()
-                env._alias_pending = False
-                env.__dict__.pop('_call_cache', None)
+                    ctypes.c_void_p(stream), env._obs_code)
+            _lib.check(env._lib.marlnav_step_host_typed(*args), "marlnav_step_host_typed")
+            env._step_launched()
             if sync:
                 torch.cuda.current_stream(env.device).synchronize()

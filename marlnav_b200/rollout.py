@@ -2,8 +2,7 @@
 
 * ``FusedActor``          -- the reference's ``Actor.forward`` + ``dist.sample()`` +
                              ``dist.log_prob()`` (/root/reference/marlnav/models.py:27-36,113-115)
-                             as one kernel launch (``marlnav_actor_sample_f32``, or
-                             ``marlnav_actor_sample_typed`` for float16 / bfloat16 observations).
+                             as one kernel launch (``marlnav_actor_sample_typed``).
 * ``discounted_returns``  -- the backward scan of ``MAPPO._process_rewards``
                              (models.py:131-139) as one kernel (``marlnav_discounted_returns_f64``),
                              optionally followed by its std/mean normalisation (models.py:141-145).
@@ -143,10 +142,7 @@ class FusedActor:
             args = (n, self.obs_size, self.hidden, p(self.w1), p(self.b1), p(self.w_mu), p(self.b_mu),
                     p(self.w_std), p(self.b_std), p(eps), self.seed, counter, p(self._counter_dev), int(row_offset),
                     p(actions), p(log_probs), p(mu), p(var), stream)
-            if code == 0:
-                _rollout_check(self._lib.marlnav_actor_sample_f32(p(x), *args), "marlnav_actor_sample_f32")
-            else:
-                _rollout_check(self._lib.marlnav_actor_sample_typed(p(x), code, *args), "marlnav_actor_sample_typed")
+            _rollout_check(self._lib.marlnav_actor_sample_typed(p(x), code, *args), "marlnav_actor_sample_typed")
         return (actions, log_probs, mu, var) if want_moments else (actions, log_probs)
 
 
@@ -188,11 +184,7 @@ class FusedCritic:
             args = (x.shape[0], self.inputs, self.hidden, self.w1.data_ptr(), self.b1.data_ptr(),
                     self.w2.data_ptr(), self.b2.data_ptr(), v.data_ptr(),
                     torch.cuda.current_stream(self.device).cuda_stream)
-            if code == 0:
-                _rollout_check(self._lib.marlnav_critic_value_f32(x.data_ptr(), *args), "marlnav_critic_value_f32")
-            else:
-                _rollout_check(self._lib.marlnav_critic_value_typed(x.data_ptr(), code, *args),
-                               "marlnav_critic_value_typed")
+            _rollout_check(self._lib.marlnav_critic_value_typed(x.data_ptr(), code, *args), "marlnav_critic_value_typed")
         return v
 
 
@@ -255,7 +247,7 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
     ``obs (T,B,A,S)``, ``actions (T,B*A,2)``, ``log_probs (T,B*A)``, ``rewards (T,B)``, ``done (T,B)``
     and ``values (T,B,1)`` when a critic is given.
 
-    ``fuse_actor``: sample the actions inside the step launch (``marlnav_act_step_f32``: one launch
+    ``fuse_actor``: sample the actions inside the step launch (``marlnav_act_step_typed``: one launch
     per iteration instead of two) where that kernel exists -- 3 agents, 1..6 obstacles; same bits
     either way (``test_fused_actor_step_matches_two_launches``).
 

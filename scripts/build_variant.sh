@@ -1,5 +1,5 @@
 #!/bin/bash
-# build_ab/lib<NAME>.so with extra nvcc flags:  scripts/build_variant.sh S0 "-DMN_TEAM_SHARE=0"
+# build_ab/lib<NAME>.so with extra nvcc flags:  scripts/build_variant.sh R64 "-maxrregcount=64"
 set -e
 mkdir -p build_ab
 nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -fmad=false -prec-div=true -prec-sqrt=true -ftz=false \
