@@ -290,8 +290,10 @@ const char* marlnav_rollout_last_error(void);
 }
 #endif
 
-/* float16 / bfloat16 observations: the `_typed` entry points of the step, then of the rollout */
+/* float16 / bfloat16 observations: the `_typed` entry points of the step, then of the rollout;
+ * final observations of auto-reset envs and truncation-aware GAE */
 #include "marlnav_b200_typed.h"
 #include "marlnav_b200_rollout_typed.h"
+#include "marlnav_b200_final.h"
 
 #endif /* MARLNAV_B200_H */

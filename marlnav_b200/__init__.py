@@ -6,11 +6,11 @@ from ._lib import MarlnavError, LIB_PATH          # noqa: F401
 from .env import Env, HostStepper, Observations, split_observations   # noqa: F401
 from .params import default_env_params, template_env_params, ring_template   # noqa: F401
 from .rollout import (FusedActor, FusedCritic, MappoRollout, RolloutGraph, StepGraph,   # noqa: F401
-                      discounted_returns, collect_rollout)
+                      discounted_returns, gae, collect_rollout)
 from .sharding import shard_bounds, shard_env_params, reduce_episode_stats, global_episode_stats  # noqa: F401
 
 __all__ = ["Env", "HostStepper", "Observations", "split_observations", "default_env_params",
            "template_env_params", "ring_template", "shard_bounds", "shard_env_params",
            "reduce_episode_stats", "global_episode_stats", "MarlnavError", "LIB_PATH",
            "FusedActor", "FusedCritic", "MappoRollout", "RolloutGraph", "StepGraph", "discounted_returns",
-           "collect_rollout"]
+           "gae", "collect_rollout"]

@@ -26,6 +26,9 @@ TYPED_EXPORTS = ("marlnav_observe_typed", "marlnav_step_typed", "marlnav_step_ca
 # every symbol include/marlnav_b200_rollout_typed.h declares (16-bit observations into the actor, the
 # critic and the fused actor+step; included by marlnav_b200.h)
 ROLLOUT_TYPED_EXPORTS = ("marlnav_actor_sample_typed", "marlnav_critic_value_typed", "marlnav_act_step_typed")
+# every symbol include/marlnav_b200_final.h declares (final observations of auto-reset envs and the
+# truncation-aware GAE scan; included by marlnav_b200.h)
+FINAL_EXPORTS = ("marlnav_step_final_typed", "marlnav_step_call_final_typed", "marlnav_gae_f64")
 
 
 class _Sized(ctypes.Structure):
@@ -110,7 +113,7 @@ def load():
     lib.marlnav_rollout_last_error.restype = ctypes.c_char_p
     sizeofs = ("marlnav_sizeof_env_params", "marlnav_sizeof_reset_spec", "marlnav_sizeof_io_transform",
                "marlnav_sizeof_actor_spec", "marlnav_sizeof_step_call")
-    for name in EXPORTS + TYPED_EXPORTS + ROLLOUT_TYPED_EXPORTS:
+    for name in EXPORTS + TYPED_EXPORTS + ROLLOUT_TYPED_EXPORTS + FINAL_EXPORTS:
         if name in sizeofs:
             getattr(lib, name).restype = ctypes.c_size_t
         elif name == "marlnav_host_pipe_destroy":
@@ -139,6 +142,9 @@ def load():
     lib.marlnav_actor_sample_typed.argtypes = [vp, i32, i64, i32, i32] + [vp] * 7 + [u64, u64, vp, u64] + [vp] * 5
     lib.marlnav_critic_value_typed.argtypes = [vp, i32, i64, i32, i32] + [vp] * 6
     lib.marlnav_act_step_typed.argtypes = [vp] * 12 + [i32] + [vp] * 6
+    lib.marlnav_step_final_typed.argtypes = [vp] * 9 + [i32] + [vp] * 7
+    lib.marlnav_step_call_final_typed.argtypes = [vp, i32, vp]
+    lib.marlnav_gae_f64.argtypes = [vp] * 6 + [f64, f64, i32, i64, vp, vp, vp]
     got = lib.marlnav_abi_version()
     if got != ABI_VERSION:
         raise MarlnavError(f"libmarlnav_b200.so ABI {got} != binding ABI {ABI_VERSION}; rebuild")

@@ -17,7 +17,8 @@ DEPS = [SRC, SRC2, os.path.join(_HERE, "csrc", "marlnav_math.cuh"), os.path.join
         os.path.join(_HERE, "csrc", "marlnav_launch.cuh"),
         os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200.h"),
         os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_typed.h"),
-        os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_rollout_typed.h")]
+        os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_rollout_typed.h"),
+        os.path.join(os.path.dirname(_HERE), "include", "marlnav_b200_final.h")]
 LIB = os.path.join(_HERE, "libmarlnav_b200.so")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -192,6 +192,50 @@ __global__ void discounted_returns_kernel(const float* __restrict__ rewards, con
     }
 }
 
+// Generalised advantage estimation that tells a time-limit truncation (bootstrapped from the
+// value of the observation the episode ended on) from a termination (include/marlnav_b200_final.h),
+// in float64 with every operation rounded to nearest and no FMA.  Shaped like
+// discounted_returns_kernel: a thread per env, the loads eight steps ahead of the recurrence.
+__global__ void gae_kernel(const float* __restrict__ rewards, const float* __restrict__ values,
+                           const uint8_t* __restrict__ terminated, const uint8_t* __restrict__ truncated,
+                           const float* __restrict__ final_values, const float* __restrict__ last_values,
+                           double gamma, double lam, int T, long long B, double* __restrict__ adv_out,
+                           double* __restrict__ ret_out) {
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const double gl = __dmul_rn(gamma, lam);
+    double adv = 0.0;
+    double v_next = last_values ? (double)last_values[b] : 0.0;     // values[t+1, b]
+    const auto step = [&](long long i, float r, float v, uint8_t te, uint8_t tr, float fv) {
+        const double vd = (double)v;
+        double nv = v_next;
+        bool cont = true;
+        if (te) { nv = 0.0; cont = false; }
+        else if (tr) { nv = (double)fv; cont = false; }
+        const double delta = __dsub_rn(__dadd_rn((double)r, __dmul_rn(gamma, nv)), vd);
+        adv = cont ? __dadd_rn(delta, __dmul_rn(gl, adv)) : delta;
+        adv_out[i] = adv;
+        ret_out[i] = __dadd_rn(adv, vd);
+        v_next = vd;
+    };
+    int t = T - 1;
+    for (; t >= 7; t -= 8) {
+        float r[8], v[8], fv[8]; uint8_t te[8], tr[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            const long long i = (long long)(t - u) * B + b;
+            r[u] = rewards[i]; v[u] = values[i]; te[u] = terminated[i]; tr[u] = truncated[i];
+            fv[u] = final_values ? final_values[i] : 0.f;
+        }
+#pragma unroll
+        for (int u = 0; u < 8; ++u) step((long long)(t - u) * B + b, r[u], v[u], te[u], tr[u], fv[u]);
+    }
+    for (; t >= 0; --t) {
+        const long long i = (long long)t * B + b;
+        step(i, rewards[i], values[i], terminated[i], truncated[i], final_values ? final_values[i] : 0.f);
+    }
+}
+
 }  // namespace mnr
 
 namespace {
@@ -370,6 +414,25 @@ int marlnav_discounted_returns_f64(const float* rewards, const uint8_t* done, do
         rewards, done, gamma, T, B, out);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : cuda_fail(e, "discounted_returns launch");
+}
+
+int marlnav_gae_f64(const float* rewards, const float* values, const uint8_t* terminated,
+                    const uint8_t* truncated, const float* final_values, const float* last_values,
+                    double gamma, double lam, int T, long long B,
+                    double* advantages, double* returns, void* stream) {
+    if (!rewards || !values || !terminated || !truncated || !advantages || !returns || T < 1 || B < 1) {
+        snprintf(g_err2, sizeof g_err2, "marlnav_gae_f64: NULL pointer or empty buffer");
+        return MARLNAV_ERR_BAD_ARG;
+    }
+    if (advantages == returns) {
+        snprintf(g_err2, sizeof g_err2, "marlnav_gae_f64: advantages and returns must be different buffers");
+        return MARLNAV_ERR_BAD_ARG;
+    }
+    const int threads = 128;
+    mnr::gae_kernel<<<(unsigned)((B + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
+        rewards, values, terminated, truncated, final_values, last_values, gamma, lam, T, B, advantages, returns);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : cuda_fail(e, "gae launch");
 }
 
 }  // extern "C"

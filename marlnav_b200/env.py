@@ -518,9 +518,10 @@ class Env(object):
         call.io = ctypes.addressof(self._io) if self._io is not None else None
         return call
 
-    def _launch_step(self, actions, ptrs, slot=None, stream=None):
+    def _launch_step(self, actions, ptrs, slot=None, stream=None, final_ptr=None):
         """One fused step launch writing to the four output pointers `ptrs` (or to `slot`'s), on
-        `stream` (raw handle of the current stream of this env's device; None = look it up)."""
+        `stream` (raw handle of the current stream of this env's device; None = look it up);
+        with `final_ptr` the finished envs' pre-reset observations go there too."""
         if actions.device != self.device or actions.dtype != torch.float32 or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.float32).contiguous()
         if actions.numel() != self._n_action_floats:
@@ -528,7 +529,7 @@ class Env(object):
         if stream is None:
             if torch.cuda.current_device() != self._dev_index:
                 with torch.cuda.device(self.device):
-                    return self._launch_step(actions, ptrs, slot)
+                    return self._launch_step(actions, ptrs, slot, final_ptr=final_ptr)
             stream = self._raw_stream()
         c = self._step_call_cache()
         if slot is not None:
@@ -550,16 +551,40 @@ class Env(object):
             rs.alias_first_step = 1
         call.actions = actions.data_ptr()
         call.stream = stream
-        rc = self._lib.marlnav_step_call_typed(ctypes.addressof(call), self._obs_code)
-        if rc:
-            _lib.check(rc, "marlnav_step_call_typed")
+        if final_ptr is None:
+            rc = self._lib.marlnav_step_call_typed(ctypes.addressof(call), self._obs_code)
+            if rc:
+                _lib.check(rc, "marlnav_step_call_typed")
+        else:
+            rc = self._lib.marlnav_step_call_final_typed(ctypes.addressof(call), self._obs_code, final_ptr)
+            if rc:
+                _lib.check(rc, "marlnav_step_call_final_typed")
         self._step_launched()
 
-    def step_fused(self, actions, out=None):
+    def _final_obs_ptr(self, final_obs, out):
+        n = self.num_parallel * self.num_agents * self.obs_size
+        if not isinstance(final_obs, torch.Tensor) or final_obs.device != self.device \
+                or final_obs.dtype != self.obs_dtype or final_obs.numel() < n or not final_obs.is_contiguous():
+            got = (f"{final_obs.dtype} with {final_obs.numel()} elements on {final_obs.device}"
+                   if isinstance(final_obs, torch.Tensor) else type(final_obs).__name__)
+            raise _lib.MarlnavError(f"step_fused: final_obs must be a contiguous {self.obs_dtype} tensor on "
+                                    f"{self.device} with at least {n} elements, got {got}")
+        if out is not None and final_obs.data_ptr() == out[0].data_ptr():
+            raise _lib.MarlnavError("step_fused: final_obs and out[0] must be different buffers")
+        return final_obs.data_ptr()
+
+    def step_fused(self, actions, out=None, final_obs=None):
         """One fused step.  Returns ``(obs (B,A,S), rewards (B), terminated (B) bool,
         truncated (B) bool)``; ``out`` may supply preallocated (obs, rewards,
         terminated_u8, truncated_u8) tensors to write into; ``obs`` must have the env's
-        ``obs_dtype`` and at least B*A*S elements."""
+        ``obs_dtype`` and at least B*A*S elements.
+
+        ``final_obs`` (a (B,A,S) tensor of the env's ``obs_dtype`` on its device, not ``out[0]``)
+        also receives, for every env this step finishes (terminated or truncated), the
+        observations its rewards and flags were computed from, before the auto-reset replaced them
+        (gymnasium's ``final_obs``): the bits a non-resetting env gets in ``obs``.  Rows of the
+        other envs are left as they were."""
+        final_ptr = None if final_obs is None else self._final_obs_ptr(final_obs, out)
         if out is not None:
             obs, rew, term, trunc = out
             if obs.dtype != self.obs_dtype or obs.numel() < self.num_parallel * self.num_agents * self.obs_size:
@@ -567,10 +592,11 @@ class Env(object):
                     f"step_fused: out[0] must be {self.obs_dtype} with at least "
                     f"{self.num_parallel * self.num_agents * self.obs_size} elements, got {obs.dtype} "
                     f"with {obs.numel()}")
-            self._launch_step(actions, (obs.data_ptr(), rew.data_ptr(), term.data_ptr(), trunc.data_ptr()))
+            self._launch_step(actions, (obs.data_ptr(), rew.data_ptr(), term.data_ptr(), trunc.data_ptr()),
+                              final_ptr=final_ptr)
             return obs, rew, term.view(torch.bool), trunc.view(torch.bool)
         slot, stream = self._take_slot()
-        self._launch_step(actions, None, slot, stream)
+        self._launch_step(actions, None, slot, stream, final_ptr)
         return slot['obs'], slot['rew'], slot['term'], slot['trunc']
 
     def step(self, actions):

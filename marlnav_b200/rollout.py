@@ -6,6 +6,8 @@
 * ``discounted_returns``  -- the backward scan of ``MAPPO._process_rewards``
                              (models.py:131-139) as one kernel (``marlnav_discounted_returns_f64``),
                              optionally followed by its std/mean normalisation (models.py:141-145).
+* ``gae``                 -- generalised advantage estimation that bootstraps time-limit truncations
+                             from the final observations' values (``marlnav_gae_f64``).
 * ``collect_rollout``     -- ``MAPPO.get_data`` (models.py:106-129) with device-resident (T, ...)
                              buffers instead of a Python list of lists: per step one actor launch and
                              one fused environment step (normaliser and action scaler folded in); the
@@ -219,6 +221,54 @@ def discounted_returns(rewards, done, gamma, normalize=False):
     return out
 
 
+def gae(rewards, values, terminated, truncated, gamma, lam, final_values=None, last_values=None):
+    """Generalised advantage estimation that tells a time-limit truncation from a termination, as one
+    kernel (``marlnav_gae_f64``).  Returns ``(advantages, returns)``, both (T,B) float64.
+
+    ``rewards``, ``values`` (T,B) float32 (``values`` may be (T,B,1), e.g. ``collect_rollout``'s);
+    ``terminated``, ``truncated`` (T,B) bool/uint8; ``final_values`` (T,B) or (T,B,1): the value of the
+    observation an episode was cut off on (``collect_rollout(final_obs=True)``'s), read where
+    ``truncated & ~terminated`` (None: 0); ``last_values`` (B,) or (B,1): the value of the state after
+    the last step (None: 0).  Backwards over t, per env, with ``gl = gamma * lam``::
+
+        nv = last_values if t == T-1 else values[t+1]
+        terminated: nv = 0, cont = 0;  truncated: nv = final_values[t], cont = 0;  else cont = 1
+        delta = (r + gamma*nv) - v;  adv = delta + gl*adv_next if cont else delta;  ret = adv + v
+
+    Every operation is a float64 operation rounded to nearest, without fused multiply-adds."""
+    lib = _lib.load()
+    if rewards.device.type != 'cuda':
+        raise _lib.MarlnavError("gae needs CUDA tensors (no CPU fallback)")
+    if rewards.dim() != 2:
+        raise _lib.MarlnavError(f"gae: rewards must be (T,B), got {tuple(rewards.shape)}")
+    T, B = rewards.shape
+    dev = rewards.device
+
+    def f32(t, n, name):
+        if t.numel() != n:
+            raise _lib.MarlnavError(f"gae: {name} must hold {n} values (T = {T}, B = {B}), got {tuple(t.shape)}")
+        return t.to(device=dev, dtype=torch.float32).reshape(-1).contiguous()
+
+    def u8(t, name):
+        if tuple(t.shape) != (T, B):
+            raise _lib.MarlnavError(f"gae: {name} must be (T,B) = ({T}, {B}), got {tuple(t.shape)}")
+        t = t.to(dev)
+        return (t.view(torch.uint8) if t.dtype == torch.bool else (t != 0).to(torch.uint8)).contiguous()
+
+    r, v = f32(rewards, T * B, 'rewards'), f32(values, T * B, 'values')
+    te, tr = u8(terminated, 'terminated'), u8(truncated, 'truncated')
+    fv = f32(final_values, T * B, 'final_values') if final_values is not None else None
+    lv = f32(last_values, B, 'last_values') if last_values is not None else None
+    p = lambda t: t.data_ptr() if t is not None else None
+    with torch.cuda.device(dev):
+        adv = torch.empty(T, B, dtype=torch.float64, device=dev)
+        ret = torch.empty(T, B, dtype=torch.float64, device=dev)
+        _rollout_check(lib.marlnav_gae_f64(p(r), p(v), p(te), p(tr), p(fv), p(lv), float(gamma), float(lam),
+                                           int(T), int(B), p(adv), p(ret), torch.cuda.current_stream(dev).cuda_stream),
+                       "marlnav_gae_f64")
+    return adv, ret
+
+
 def _require_obs_dtype(env, obs_dtype, what):
     """A rollout's observation buffer has the type the caller asked for, and it must be the env's: a
     16-bit buffer goes to a learner, whose float32 layers refuse it unless it casts, so a 16-bit env
@@ -237,7 +287,7 @@ def _require_f32_obs(env, what):
 
 @torch.no_grad()
 def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None, scaler_params=None,
-                    fuse_actor=True, obs_dtype=torch.float32):
+                    fuse_actor=True, obs_dtype=torch.float32, final_obs=False):
     """``MAPPO.get_data`` (models.py:106-129) on device-resident buffers.
 
     ``env``: a ``marlnav_b200.Env``; ``actor``: a ``FusedActor``; ``critic``: optional ``FusedCritic``
@@ -255,7 +305,15 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
     With ``torch.float16`` / ``torch.bfloat16`` every stored observation is the normalised float32
     value rounded to nearest-even (``obs32.to(obs_dtype)``), and the actor and a ``FusedCritic`` read
     those values widened exactly to float32; a torch-module critic gets ``obs.float()``.  Every other
-    buffer stays float32 (``done``: bool).  Cast learner minibatches with ``.float()``."""
+    buffer stays float32 (``done``: bool).  Cast learner minibatches with ``.float()``.
+
+    ``final_obs=True`` also returns, for a learner that bootstraps time-limit truncations (``gae``):
+    ``final_obs (T,B,A,S)`` in ``obs_dtype``, where row ``[t,b]`` holds the observations env b's episode
+    ended on at step t (valid where ``done[t,b]``, unspecified elsewhere), ``terminated`` and
+    ``truncated`` (T,B) bool, and with a ``FusedCritic`` ``final_values (T,B,1)``, the critic on every
+    ``final_obs`` row in one launch after the loop.  The fused actor+step kernels have no final
+    observations, so this mode runs the actor and ``step_fused`` as two launches per step, with the
+    same actions and outputs."""
     _require_obs_dtype(env, obs_dtype, "collect_rollout")
     if normalizer_params is not None or scaler_params is not None:
         env.fuse_io(normalizer_params, scaler_params)
@@ -273,6 +331,7 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
                rewards=torch.empty(T, B, device=dev))
     if critic is not None:
         buf['values'] = torch.empty(T, B, 1, device=dev)
+    fin = torch.empty(T, B, A, S, dtype=obs_dtype, device=dev) if final_obs else None
     # models.py:110; a 16-bit buffer receives the float32 quotient rounded to nearest-even
     torch.div(env._observations_f32() - mean, scale, out=obs_all[0])
     # device-resident counters: each step passes its offset, ONE add per counter after the loop
@@ -282,7 +341,7 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
     # actor -> step critical path (in a captured graph: a parallel branch joined at the end).
     main = torch.cuda.current_stream(dev)
     side = _critic_stream(dev) if isinstance(critic, FusedCritic) else None
-    fused = bool(fuse_actor) and env.supports_fused_actor(actor)
+    fused = bool(fuse_actor) and not final_obs and env.supports_fused_actor(actor)
     try:
         for t in range(T):
             obs = obs_all[t]
@@ -302,7 +361,8 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
             actions, _ = actor.act(obs, out=(buf['actions'][t], buf['log_probs'][t]),     # models.py:113-115
                                    row_offset=actor.row_offset if actor.row_offset is not None else env._env_id_offset * A)
             # raw [-1,1] actions in, normalised next observations out (models.py:116-118,122)
-            env.step_fused(actions.view(B, A, 2), out=(obs_all[t + 1], buf['rewards'][t], term[t], trunc[t]))
+            env.step_fused(actions.view(B, A, 2), out=(obs_all[t + 1], buf['rewards'][t], term[t], trunc[t]),
+                           final_obs=None if fin is None else fin[t])
     finally:
         if side is not None:
             main.wait_stream(side)
@@ -311,6 +371,12 @@ def collect_rollout(env, actor, buffer_len, critic=None, normalizer_params=None,
     buf['obs'] = obs_all[:T]
     buf['last_obs'] = obs_all[T]
     buf['done'] = torch.logical_or(term.view(torch.bool), trunc.view(torch.bool))   # models.py:119
+    if fin is not None:
+        buf['final_obs'] = fin
+        buf['terminated'], buf['truncated'] = term.view(torch.bool), trunc.view(torch.bool)
+        if isinstance(critic, FusedCritic):
+            buf['final_values'] = torch.empty(T, B, 1, device=dev)
+            critic(fin.view(T * B, A * S), out=buf['final_values'].view(T * B, 1))
     return buf
 
 
@@ -320,9 +386,10 @@ class RolloutGraph:
     sampling counter live in device memory, so every replay continues the same random streams an
     eager loop would use; ``FusedActor.refresh`` / ``FusedCritic.refresh`` update weights in place.
     ``replay()`` returns the SAME buffer tensors every time (clone what must outlive the next replay).
-    ``obs_dtype``: the observation buffer's element type, as in ``collect_rollout``."""
+    ``obs_dtype`` and ``final_obs``: as in ``collect_rollout``."""
 
-    def __init__(self, env, actor, buffer_len, critic=None, warmup_steps=2, obs_dtype=torch.float32):
+    def __init__(self, env, actor, buffer_len, critic=None, warmup_steps=2, obs_dtype=torch.float32,
+                 final_obs=False):
         _require_obs_dtype(env, obs_dtype, "RolloutGraph")
         if critic is not None and not isinstance(critic, FusedCritic):
             raise _lib.MarlnavError("RolloutGraph needs a FusedCritic (or no critic)")
@@ -334,11 +401,12 @@ class RolloutGraph:
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
             if warmup_steps:                                  # lazy kernel attributes, allocator warm-up
-                collect_rollout(env, actor, warmup_steps, critic=critic, obs_dtype=obs_dtype)
+                collect_rollout(env, actor, warmup_steps, critic=critic, obs_dtype=obs_dtype, final_obs=final_obs)
             side.synchronize()
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph, stream=side):
-                self.buffers = collect_rollout(env, actor, self.buffer_len, critic=critic, obs_dtype=obs_dtype)
+                self.buffers = collect_rollout(env, actor, self.buffer_len, critic=critic, obs_dtype=obs_dtype,
+                                               final_obs=final_obs)
         torch.cuda.current_stream(dev).wait_stream(side)
 
     def replay(self):
