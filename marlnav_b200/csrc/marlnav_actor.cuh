@@ -3,7 +3,7 @@
 // One row of the reference's Actor (/root/reference/marlnav/models.py:27-36) with its
 // diagonal-Gaussian sample and log-prob (models.py:113-115), as ONE device function shared by
 // the stand-alone actor kernel (marlnav_rollout.cu) and the fused {actor -> step} kernel
-// (marlnav_kernels.cu), so that both produce the same bits:
+// (marlnav_step_env.cu, marlnav_step_team.cu), so that both produce the same bits:
 //
 //   h = fc1(x)  (NO activation, models.py:29-31);  mu = tanh(fc_mu(h));  var = softplus(fc_std(h))
 //   dist = MultivariateNormal(mu, covariance_matrix=diag(var))   -> std dev = sqrt(var)

@@ -1,6 +1,7 @@
 // marlnav_b200/csrc/marlnav_launch.cuh
 //
-// Host-side launch set-up shared by marlnav_kernels.cu and marlnav_rollout.cu.
+// Host-side launch set-up shared by the library's units: marlnav_rollout.cu and the
+// step library (marlnav_abi.cu, marlnav_step_*.cu, marlnav_step_launch.cuh).
 #pragma once
 
 #include <cuda_runtime.h>

@@ -14,7 +14,7 @@ reference's callers touch (SURVEY.md section 8b):
     ._risk_factor ... ._bond_factor   (read by check_rews, utils.py:648-653)
 
 but ``step`` is ONE launch of the fused sm_100a kernel in
-``csrc/marlnav_kernels.cu`` through the C ABI of ``include/marlnav_b200.h``.
+``csrc/marlnav_step_*.cu`` through the C ABI of ``include/marlnav_b200.h``.
 State tensors stay resident in HBM and are updated in place; outputs are fresh
 tensors every step (the rollout buffer keeps references to them, models.py:121).
 

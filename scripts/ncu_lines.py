@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Rank the source lines of the first kernel in an .ncu-rep by executed warp instructions (per CTA).
 usage: python scripts/ncu_lines.py rep.ncu-rep [top_n]"""
-import csv, io, subprocess, sys
+import csv, io, re, subprocess, sys
 rep = sys.argv[1]; top = int(sys.argv[2]) if len(sys.argv) > 2 else 60
 src = subprocess.run(['ncu', '-i', rep, '--page', 'source', '--csv', '--print-source', 'cuda,sass'], capture_output=True, text=True).stdout
 rows = list(csv.reader(io.StringIO(src)))
@@ -14,7 +14,7 @@ per = []
 first = names[0]
 grid = None
 for n, h0 in enumerate(hi):
-    if n > 0 and rows[h0 - 2][0] == 'File Path' and rows[h0 - 2][1].endswith('marlnav_kernels.cu') and n > 0 and per: break
+    if n > 0 and rows[h0 - 2][0] == 'File Path' and re.search(r'csrc/marlnav_[a-z_]+\.cu$', rows[h0 - 2][1]) and n > 0 and per: break
     h = rows[h0]; ix = {nm: i for i, nm in enumerate(h)}
     end = hi[n + 1] - 2 if n + 1 < len(hi) else len(rows)
     fname = rows[h0 - 2][1].split('/')[-1].replace('marlnav_', '')
