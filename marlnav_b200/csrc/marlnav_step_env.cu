@@ -23,9 +23,14 @@ namespace mn {
 // What the B200 measurements (1M x 3 x 3) decided -- all variants bit-identical, see DESIGN.md 5:
 //   * one-warp CTAs: a CTA's registers and shared memory are only released when its slowest warp
 //     is done, and the tail of the last wave shrinks: 4-warp 82.0 us, 2-warp 80.2, 1-warp 78.8;
-//   * the agent loop stays ROLLED.  Unrolling it and sharing every unordered agent pair's geometry
-//     between both agents removes 15 % of the instructions but the hot path then exceeds the
-//     32 KB L1.5 instruction cache (stall_no_inst 10 % -> 18 %): 83.2 us, no gain;
+//   * P2 is split in two blocks, each smaller than the one rolled agent-loop body it replaces
+//     (368 instructions at (3,3)): P2a, straight-line, evaluates each unordered agent pair ONCE for
+//     both agents (geometry, bond quotient, compares; only the angle is taken per direction); P2b,
+//     rolled over the team, takes the target and the obstacles.  P2a hands each agent's bond term to
+//     P2b through the lane's dead obstacle / target tile slots and its flags and pair count through
+//     one register of bit fields: no local memory, no larger tile.  (Unrolling the whole team
+//     instead removes 15 % of the instructions but the hot path then exceeds the 32 KB L1.5
+//     instruction cache, stall_no_inst 10 % -> 18 %: 83.2 us, no gain.);
 //   * persistent warps with double-buffered TMA prefetch (91-121 us) and observation rows stored
 //     straight from registers with 256-bit STG (86 us) both lost to this layout;
 //   * one range test per env (min |component|, max d^2 over all its pairs, NaN-propagating)
@@ -52,19 +57,80 @@ struct EnvTile {
     static constexpr bool kRowVec = S % 4 == 0;     // float4 row stores into the tile (odd obstacle counts)
     static constexpr size_t smem_bytes() { return (size_t)BYTES + 8; }
     // resident CTAs per SM the compiler schedules for.  Shared memory, not registers, bounds the
-    // occupancy (26 CTAs/SM at (3,3), 59-64 registers either way); a looser bound lets ptxas schedule
-    // better: measured at 1M x 3 x 3 on B200, 28: 66.5 us, 24: 66.45, 20: 66.3, 16 / 12 / 8: 65.85.
-    static constexpr int CTAS = 16;
+    // occupancy (26 CTAs/SM at (3,3), 55-64 registers either way); a looser bound lets ptxas schedule
+    // better: measured at 1M x 3 x 3 on B200, 28: 66.5 us, 24: 66.45, 20: 66.3, 16 / 12 / 8: 65.85
+    // with one rolled agent loop; with the split P2, 26: 65.7, 16: 64.26, 8: 63.81 (medians of 6;
+    // 4 and 1 give the same code as 8).
+    static constexpr int CTAS = 8;
 };
 
-// One agent against its N = 1 + O + R objects on the branch-free fast path (see pair_obs), the
-// agent's own state and the other agents read from the env's shared-memory row.
+// Where P2a leaves each agent's bond term for P2b: this lane's obstacle / target slots of the tile,
+// dead once P2 holds them in registers (P4a rewrites them from registers for the envs it resets
+// before P4b reads them, P5 never stores them, the guarded fallback takes them from registers).
+// 2 * O + 2 >= A slots for every O >= 1.
+template <int A, int O>
+__device__ __forceinline__ float* bond_slot(float* ob_env, float* tg_env, int a) {
+    static_assert(2 * O + 2 >= A, "slots");
+    if constexpr (2 * O >= A) return ob_env + a;
+    else return a < 2 * O ? ob_env + a : tg_env + (a - 2 * O);
+}
+
+// P2a: every agent pair of the env once, on the branch-free fast path (see pair_obs), straight-line.
+// For i < j the geometry of (i -> j) serves (j -> i) as well: on the fast path every component is
+// non-zero, so cdist(j, i) == cdist(i, j) and normalize(i - j) is exactly -normalize(j - i); only
+// the angle, taken against each agent's own heading, is evaluated per direction.  The bond quotient
+// and the compares depend on the distance alone.  Writes the others' columns of every agent's row
+// and leaves, per agent a, its bond term in bond_slot(a) and in `flags` bits 4a..4a+3: ag_risk,
+// ag_coll and the count of agents between agents_min_d and agents_max_d (0..R).
 template <int A, int O, class DM, bool NORM, class OT>
-__device__ __forceinline__ void observe_agent_fast(const marlnav_env_params& p, const DivConsts& rc,
-                                                   const float* __restrict__ st_env, const float (&OBX)[O],
-                                                   const float (&OBY)[O], float tx, float ty, int a,
-                                                   const ObsRow<NORM, OT>& sink, float& lo, float& dmin, AgentTerms& tm) {
-    constexpr int R = A - 1, N = 1 + O + R;
+__device__ __forceinline__ void observe_agent_pairs(const marlnav_env_params& p, const DivConsts& rc,
+                                                    const float* __restrict__ st_env, OT* obs_env,
+                                                    ObsRow<NORM, OT> sink, float* ob_env, float* tg_env,
+                                                    float& lo, float& dmin, unsigned& flags) {
+    constexpr int R = A - 1, S = EnvTile<A, O>::S;
+    static_assert(4 * A <= 32 && R <= 3, "flag bits");
+    const float cap = p.cap_distance;
+    float an[A][R > 0 ? R : 1], di[A][R > 0 ? R : 1], q[A][R > 0 ? R : 1];   // [agent][k-th other]
+    unsigned fl = 0u;
+#pragma unroll
+    for (int i = 0; i < A; ++i) {
+#pragma unroll
+        for (int j = i + 1; j < A; ++j) {
+            const int ki = j - 1, kj = i;                   // j among i's others, i among j's (:22-24)
+            float d, nx, ny;
+            geom_fast(st_env[5 * j + 0] - st_env[5 * i + 0], st_env[5 * j + 1] - st_env[5 * i + 1], d, nx, ny, lo);
+            pair_finish<false>(d, nx, ny, st_env[5 * i + 2], st_env[5 * i + 3], cap, an[i][ki], di[i][ki]);
+            pair_finish<false>(d, -nx, -ny, st_env[5 * j + 2], st_env[5 * j + 3], cap, an[j][kj], di[j][kj]);
+            dmin = fminf(dmin, d);
+            const unsigned both = (1u << (4 * i)) | (1u << (4 * j));
+            if (d < p.ag_risk_dist) fl |= both;
+            if (d < p.ag_coll_dist) fl |= both << 1;
+            if (p.agents_min_d < d && d < p.agents_max_d) fl += both << 2;
+            const float sd = div_mode<DM::kSharp, false>(d - p.ideal_dist, p.bond_sharpness, rc.sharp);
+            q[i][ki] = q[j][kj] = rcp_rn_normal(1.0f + sd * sd);
+        }
+    }
+#pragma unroll
+    for (int a = 0; a < A; ++a) {
+        float cols[2 * R];
+#pragma unroll
+        for (int k = 0; k < R; ++k) { cols[k] = an[a][k]; cols[R + k] = di[a][k]; }
+        sink.row = obs_env + a * S;
+        sink.template put_cols<2 + 2 * O, 2 * R, EnvTile<A, O>::kRowVec>(cols);
+        *bond_slot<A, O>(ob_env, tg_env, a) = div_mode<DM::kR, false>(torch_row_sum(q[a], R), (float)R, rc.R);
+    }
+    flags = fl;
+}
+
+// P2b: agent `a` against the target and the O obstacles on the fast path, the rest of its row, and
+// its reward ingredients with the agent-pair terms P2a left for it (environment.py:186-202).
+template <int A, int O, class DM, bool NORM, class OT>
+__device__ __forceinline__ void observe_agent_objects(const marlnav_env_params& p, const DivConsts& rc,
+                                                      const float* __restrict__ st_env, const float (&OBX)[O],
+                                                      const float (&OBY)[O], float tx, float ty, int a,
+                                                      const ObsRow<NORM, OT>& sink, float bond, unsigned flags,
+                                                      float& lo, float& dmin, AgentTerms& tm) {
+    constexpr int N = 1 + O;
     const float ox = st_env[5 * a + 0], oy = st_env[5 * a + 1];
     const float hx = st_env[5 * a + 2], hy = st_env[5 * a + 3];
     const float cap = p.cap_distance;
@@ -72,11 +138,6 @@ __device__ __forceinline__ void observe_agent_fast(const marlnav_env_params& p, 
     px[0] = tx; py[0] = ty;
 #pragma unroll
     for (int j = 0; j < O; ++j) { px[1 + j] = OBX[j]; py[1 + j] = OBY[j]; }
-#pragma unroll
-    for (int k = 0; k < R; ++k) {
-        const int j = k + (k >= a ? 1 : 0);                 // others in ascending index, skipping self (:22-24)
-        px[1 + O + k] = st_env[5 * j + 0]; py[1 + O + k] = st_env[5 * j + 1];
-    }
 #pragma unroll
     for (int i = 0; i < N; ++i) {
         float d, nx, ny;
@@ -86,7 +147,26 @@ __device__ __forceinline__ void observe_agent_fast(const marlnav_env_params& p, 
 #pragma unroll
     for (int i = 0; i + 1 < N; i += 2) dmin = min3f(dmin, di[i], di[i + 1]);
     if constexpr (N % 2 == 1) dmin = fminf(dmin, di[N - 1]);
-    agent_row_and_terms<O, R, true, DM>(p, rc, an, di, sink, EnvTile<A, O>::kRowVec, tm);
+    float row[2 + 2 * O];
+    row[0] = an[0]; row[1] = di[0];
+    bool ob_risk = false, ob_coll = false;
+#pragma unroll
+    for (int j = 0; j < O; ++j) {
+        row[2 + j] = an[1 + j]; row[2 + O + j] = di[1 + j];
+        ob_risk |= di[1 + j] < p.ob_risk_dist; ob_coll |= di[1 + j] < p.ob_coll_dist;
+    }
+    sink.template put_cols<0, 2 + 2 * O, EnvTile<A, O>::kRowVec>(row);
+    const unsigned f = flags >> (4 * a);
+    tm.risk = (ob_risk || (f & 1u) != 0u) ? 1.f : 0.f;
+    tm.coll = ob_coll || (f & 2u) != 0u;
+    tm.in_t = di[0] < p.target_radius;
+    const float cnt = (float)((f >> 2) & 3u);            // the reference's sum of 0/1 terms, exact
+    const float capped = cnt > p.max_at_prop_d ? p.max_at_prop_d : cnt;
+    tm.dsc = div_mode<DM::kProp, false>(capped, p.max_at_prop_d, rc.prop_d);
+    tm.head = fabsf(an[0]) < p.max_angle_diff ? 1.f : 0.f;
+    // 2^-39 < di[0] < 2^50 (the caller's range test), inside the proven sequence's range
+    tm.soft = -1.0f * div_mode<DM::kInit, true>(di[0], p.init_dist, rc.init_dist);
+    tm.bond = bond;
 }
 
 // ACTOR: the actions are not read but sampled here, from the reference's Actor applied to the
@@ -237,7 +317,7 @@ step_env_kernel(const StepArgs args) {
             for (int k = 0; k < 5; ++k) st_env[5 * a + k] = s[k] + wash;
         }
 
-        // ---- P2: observe + per-agent reward terms (rolled over the team: code size, see above)
+        // ---- P2: observe + per-agent reward terms
 #pragma unroll
         for (int j = 0; j < O; ++j) {
             const float2 ob = *reinterpret_cast<const float2*>(ob_env + 2 * j);
@@ -252,17 +332,25 @@ step_env_kernel(const StepArgs args) {
         ObsRow<NORM, OT> sink;
         sink.mean = args.io.obs_mean; sink.scale = args.io.obs_scale;
         OT* const obs_env = w_obs + lane * A * S;
+        float* const tg_env = w_tg + lane * 2;
+        unsigned pair_flags;
+        // ---- P2a: agent pairs, each once (straight-line)
+        observe_agent_pairs<A, O, DM>(p, rc, st_env, obs_env, sink, ob_env, tg_env, lo, dmin, pair_flags);
+        // ---- P2b: target and obstacles, rolled over the team (code size, see above); the reward
+        // terms summed from agent 0 up as torch does
 #pragma unroll 1
         for (int a = 0; a < A; ++a) {
             sink.row = obs_env + a * S;
             AgentTerms tm;
-            observe_agent_fast<A, O, DM>(p, rc, st_env, OBX, OBY, tg.x, tg.y, a, sink, lo, dmin, tm);
+            observe_agent_objects<A, O, DM>(p, rc, st_env, OBX, OBY, tg.x, tg.y, a, sink,
+                                            *bond_slot<A, O>(ob_env, tg_env, a), pair_flags, lo, dmin, tm);
             all_in = all_in && tm.in_t;
             coll_any = coll_any || tm.coll;
             float r_out, r_in;
             agent_reward2(p, tm, r_out, r_in);
             sum_out = sum_out + r_out; sum_in = sum_in + r_in;
         }
+        // ---- P2c: guarded fallback
         // Fast-path validity (see pair_obs, geom_fast): every |ex|, |ey| > 2^-39, every coordinate
         // below 2^48 (=> every d^2 < 2^100) and every distance >= cap (the fast path leaves the cap
         // rule out).  Anything else (exactly aligned agents, absurd magnitudes, coincident points)
