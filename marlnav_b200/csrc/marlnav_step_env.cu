@@ -196,7 +196,13 @@ step_env_kernel(const StepArgs args) {
     OT* const w_obs = reinterpret_cast<OT*>(w_tg + W::TG);
     uint64_t* const bar = reinterpret_cast<uint64_t*>(reinterpret_cast<char*>(smem_raw) + W::BYTES);
 
-    const long long wenv0 = (long long)blockIdx.x << 5;
+    // Odd steps visit the tiles in reverse (CTA i takes tile gridDim.x - 1 - i): each step starts on
+    // the tiles the previous one finished last, whose state is the likeliest to be still in L2
+    // (the parity is the host's step counter: no load before the bulk copies are issued).  The
+    // fused-actor build keeps the launch order: it steps rollouts of small, L2-resident batches, and
+    // there the reversal measured 0.8 % slower per rollout iteration at 1 024 envs.
+    const unsigned tile = (!ACTOR && (rs.step_counter & 1u)) ? gridDim.x - 1u - blockIdx.x : blockIdx.x;
+    const long long wenv0 = (long long)tile << 5;
     const long long left = (long long)p.num_envs - wenv0;
     const int nenv = left < 32 ? (int)left : 32;
     const bool bulk = args.vec_ok != 0 && nenv == 32;

@@ -272,7 +272,9 @@ step_team_kernel(const StepArgs args) {
     OT* const w_obs = reinterpret_cast<OT*>(w_tg + W::TG);
     uint64_t* const bar = reinterpret_cast<uint64_t*>(reinterpret_cast<char*>(smem_raw) + W::BYTES);
 
-    const long long wenv0 = (long long)blockIdx.x * ENVS;
+    // odd steps visit the tiles in reverse, except in the fused-actor build (see step_env_kernel)
+    const unsigned tile = (!ACTOR && (rs.step_counter & 1u)) ? gridDim.x - 1u - blockIdx.x : blockIdx.x;
+    const long long wenv0 = (long long)tile * ENVS;
     const long long left = (long long)p.num_envs - wenv0;
     const int nenv = left < ENVS ? (int)left : ENVS;
     const bool bulk = args.vec_ok != 0 && nenv == ENVS;
